@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: Gaussian x view votes/s (label lifting) and K-means iters/s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -27,10 +27,20 @@ sharded float64 update from the reference's float32 mean and from the exact mean
 `--impl reference` times the reference's CPU algorithm instead: the reference is pure Python
 and cannot be compiled, so this runs the oracle's C port of it (oracle/gsl_oracle.c, OpenMP,
 every core the process may use) on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes, after the run, what the last timed step returned, as float32 .npy
+files: lift_labels (one label per Gaussian), and kmeans_labels, kmeans_centroids, kmeans_shift
+of the last timed K-means iteration.  The inputs are seeded, so two builds run with the same
+arguments can be compared file by file.  The files stay under 64 MB: for larger workloads the
+label arrays keep the same fraction of their rows, picked by np.random.default_rng(0), in order.
+
+Nothing is written into the repository tree, which may be read-only: no bytecode, and the
+libraries are the ones `__graft_entry__.build()` compiled.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import importlib
 import json
 import os
@@ -38,6 +48,8 @@ import subprocess
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True
 
 import numpy as np
 
@@ -49,10 +61,18 @@ METRIC = "gaussian_view_votes_per_s"
 UNIT = "votes/s"
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"{s} is not a positive integer")
+    return v
+
+
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=positive_int, default=20,
+                    help="timed lifting passes, K-means iterations and end-to-end calls")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["native", "reference"], default="native")
     ap.add_argument("--gaussians", type=int, default=6_000_000)
@@ -68,6 +88,7 @@ def parse_args():
     ap.add_argument("--skip-cpu", action="store_true", help="no CPU oracle legs (parity and cpu_baseline become null)")
     ap.add_argument("--skip-kmeans", action="store_true")
     ap.add_argument("--skip-next", action="store_true", help="no section-8f rows (viewer depth sort / hit test, region-growing normals)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -83,13 +104,7 @@ def workload_config(a):
 
 
 def peak_hbm():
-    path = os.path.join(ROOT, "MEASURED_PEAKS.json")
-    if os.path.exists(path):
-        try:
-            return float(json.load(open(path))["hbm_gbs"]), "measured (MEASURED_PEAKS.json)"
-        except Exception:
-            pass
-    return 6650.0, "fallback (B200_PROFILING.md)"
+    return 6521.1, "HBM copy bandwidth measured on a B200 (DESIGN.md section 4)"
 
 
 def ncu_traffic(name, world):
@@ -118,6 +133,7 @@ class ClockSampler:
                 ["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "20", "-i", str(self.index)],
                 stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
             threading.Thread(target=self._pump, daemon=True).start()
+            atexit.register(self.stop)             # also when the run fails: no nvidia-smi left behind
         except Exception:
             self.proc = None
 
@@ -126,8 +142,9 @@ class ClockSampler:
             self.rows.append((time.time(), line.strip()))
 
     def stop(self):
-        if self.proc is not None:
+        if self.proc is not None and self.proc.poll() is None:
             self.proc.terminate()
+            self.proc.wait()
 
     def summary(self, t0, t1):
         sm, mx, reasons, power = [], [], set(), []
@@ -170,6 +187,25 @@ def build_scene(a, gs, pinned):
 def kmeans_init(a, feats):
     np.random.seed(0)
     return feats[np.random.choice(a.kmeans_rows, a.kmeans_k, replace=False)]
+
+
+DUMP_BYTES = 60_000_000          # array data; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(path, arrays):
+    """Write each array as path/<name>.npy in float32 (labels are small integers: exact).  Over
+    DUMP_BYTES in all, every array above 1 MB keeps the same fraction of its rows, a seeded
+    sorted sample; the small ones (centroids, shift) are written whole."""
+    arrays = {name: np.asarray(x, np.float32) for name, x in arrays.items()}
+    small = sum(x.nbytes for x in arrays.values() if x.nbytes <= 1 << 20)
+    big = sum(x.nbytes for x in arrays.values() if x.nbytes > 1 << 20)
+    keep = min(1.0, (DUMP_BYTES - small) / big) if big else 1.0
+    os.makedirs(path, exist_ok=True)
+    for name, x in arrays.items():
+        if keep < 1.0 and x.nbytes > 1 << 20:
+            rows = np.random.default_rng(0).choice(len(x), int(len(x) * keep), replace=False)
+            x = x[np.sort(rows)]
+        np.save(os.path.join(path, name + ".npy"), x)
 
 
 # ----------------------------------------------------------------------------------------
@@ -368,6 +404,9 @@ def run_native(a):
         ev[i].record(); run_prepare(); run_sweep()
     ev[a.steps].record()
     n_lift_launches = launches() - n_launch0
+    dump = {}
+    if a.dump_outputs:
+        lift_out = labels.clone()                  # the per-phase runs below write `labels` again
     barrier()
     t_wall1 = time.time()
     total_ms = sharding.barrier_max_ms(ev[0].elapsed_time(ev[-1]), dev)
@@ -391,6 +430,9 @@ def run_native(a):
     parity = {"lifting": None, "kmeans": None}
     cpu = None
     all_labels = sharding.gather_labels(labels, a.gaussians, rank, world)
+    if a.dump_outputs:
+        dump["lift_labels"] = sharding.gather_labels(lift_out, a.gaussians, rank, world)
+        del lift_out
     if orc is not None:
         n_s = min(a.parity_gaussians, a.gaussians)
         r, dt, vis, want, near = cpu_lift_sample(a, orc, cams, pos, maps, n_s, want_near=True)
@@ -473,18 +515,20 @@ def run_native(a):
             k_iter(d_cen)
         barrier()
         kev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
-        ksteps = max(a.steps, 5)
         cur = d_cen.clone()
         k_launch0 = launches()
         kev[0].record()
-        for _ in range(ksteps):
+        for _ in range(a.steps):
             k_iter(cur)
             cur.copy_(new_c)                       # real Lloyd iterations: centroids move
         kev[1].record()
         k_launches = launches() - k_launch0
+        if a.dump_outputs:                         # the ordered-update timing below writes k_labels again
+            dump["kmeans_centroids"], dump["kmeans_shift"] = new_c.clone(), shift.clone()
+            dump["kmeans_labels"] = sharding.gather_labels(k_labels.clone(), a.kmeans_rows, rank, world)
         barrier()
         t_k1 = time.time()
-        k_ms = sharding.barrier_max_ms(kev[0].elapsed_time(kev[1]), dev) / ksteps
+        k_ms = sharding.barrier_max_ms(kev[0].elapsed_time(kev[1]), dev) / a.steps
         peak, peak_src = peak_hbm()
         rows_r = khi - klo
         k_bytes = rows_r * (4 * a.kmeans_dim + 4) + 2 * a.kmeans_k * a.kmeans_dim * 4
@@ -493,7 +537,7 @@ def run_native(a):
                 "roofline": {"bound": "hbm", "achieved": k_bytes / (k_ms * 1e-3) / 1e9, "peak": peak, "unit": "GB/s",
                              "frac": k_bytes / (k_ms * 1e-3) / 1e9 / peak, "traffic": ncu_traffic("kmeans_step_kernel", world),
                              "algorithmic_bytes": k_bytes, "peak_source": peak_src},
-                "gpu_launches_per_iter": k_launches / ksteps}
+                "gpu_launches_per_iter": k_launches / a.steps}
         if world == 1:
             # reference-order (bit-exact) update, single device
             oev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
@@ -506,17 +550,20 @@ def run_native(a):
             oev[1].record(); torch.cuda.synchronize()
             kres["ordered_ms_per_iter"] = oev[0].elapsed_time(oev[1]) / 3
         if not a.skip_e2e:
-            for rep in range(4):                       # three warm-up calls (allocator, pinned buffers, NCCL), the fourth is timed
+            call_s = []
+            for rep in range(3 + a.steps):             # three warm-up calls (allocator, pinned buffers, NCCL), then the timed ones
                 barrier()
                 t0 = time.perf_counter()
                 dd = feats_pinned.to(dev, non_blocking=True)
                 cen_e, lab_e, it_e = km.lloyd(dd, d_cen, max_iter=5, tol=0.0, update="fast", verbose=False)
                 lab_host = dls._to_host(lab_e)
                 barrier()
-                dt = time.perf_counter() - t0
+                if rep >= 3:
+                    call_s.append(time.perf_counter() - t0)
                 del dd
-            dt = sharding.barrier_max_ms(dt * 1e3, dev) * 1e-3
-            kres["e2e"] = {"value": 5 / dt, "unit": "iters/s", "call": "k_means.lloyd(max_iter=5) incl. H2D rows + final assignment + D2H labels",
+            dt = sharding.barrier_max_ms(float(np.mean(call_s)) * 1e3, dev) * 1e-3
+            kres["e2e"] = {"value": 5 / dt, "unit": "iters/s", "calls": a.steps,
+                           "call": "k_means.lloyd(max_iter=5) incl. H2D rows + final assignment + D2H labels",
                            "h2d_bytes_per_call": int(feats_pinned.numel() * 4 * 1), "d2h_bytes_per_call": int(lab_host.size * 4)}
         if orc is not None:
             rows = min(3_000_000, a.kmeans_rows)
@@ -534,7 +581,7 @@ def run_native(a):
     if not a.skip_e2e:
         pos_pinned = torch.from_numpy(pos[lo:hi]).pin_memory()
         seg_list = [maps_pinned[v] for v in range(V)]
-        steps_e = max(2, min(a.steps, 5))
+        steps_e = a.steps
         warm_e = 3                                     # W >= 3: allocator blocks and both pinned result buffers exist
         got = None
         per_call = []
@@ -598,6 +645,8 @@ def run_native(a):
             "clocks": clocks, "clocks_window": "lifting + k-means timed regions, nvidia-smi -lms 20", "label_histogram_head": label_hist,
         }
         print(json.dumps(line))
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, {name: t.cpu().numpy() for name, t in dump.items()})
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -606,6 +655,8 @@ def run_native(a):
 def main():
     a = parse_args()
     if a.impl == "reference":
+        if a.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs writes what the native arm computed; it has no meaning with --impl reference")
         run_reference(a)
     else:
         run_native(a)
