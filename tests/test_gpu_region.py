@@ -7,7 +7,8 @@ Bars (floating point, stated here):
     (eigenvalue gap > 1e-2 of the largest), same orientation unless the point lies on its own plane
   * residuals: absolute 1e-5 of a cloud ~4 units wide (the reference's centroid is a float32
     sequential mean, the GPU's a float64 sum: ~1e-7); 1e-6 with the reference's normals handed in
-  * segmentation_3D: the same partition into regions as the reference."""
+  * segmentation_3D: the same partition into regions as the reference.
+The exact neighbour sets for k > 64 are checked against a float64 reference in test_region_exact_sets.py."""
 import contextlib
 import io
 import os
@@ -16,7 +17,7 @@ import numpy as np
 import pytest
 import torch
 
-from util import GOLDEN, pkg
+from util import GOLDEN, blobs, pkg
 
 pytestmark = pytest.mark.gpu
 
@@ -74,16 +75,11 @@ def test_golden_cases_through_the_mirror(oracle, name):
     assert len(set(zip(mine.tolist(), g["region_of"].tolist()))) == len(regions)
 
 
-def _blobs(rng, n, spread=0.3):
-    centres = rng.uniform(-2, 2, size=(10, 3))
-    return (centres[rng.integers(0, 10, n)] + rng.normal(0, spread, size=(n, 3))).astype(np.float32)
-
-
 @pytest.mark.parametrize("n, k", [(5000, 1), (5000, 10), (20_000, 64), (20_000, 2000), (3000, 3000), (40, 7), (33, 33)])
 def test_random_clouds_equal_oracle(oracle, n, k):
     rg = pkg("region_growing")
     rng = np.random.default_rng(n + k)
-    pos = _blobs(rng, n)
+    pos = blobs(rng, n)
     ref = oracle.region_knn_pca(pos, k, want_knn=k <= 64)
     got = rg.knn_pca(pos, k, want_centroids=True, want_knn=k <= 64)
     if k <= 64:
@@ -109,7 +105,7 @@ def test_outliers_duplicates_and_degenerate_sets(oracle):
         scale = np.abs(ref["centroids"]).max(1) + 1
         assert (np.abs(got["centroids"].cpu().numpy() - ref["centroids"]).max(1) / scale).max() < 1e-5
     # duplicated points: exact distance ties at the k-th neighbour go to the lower index on both sides
-    base = _blobs(rng, 500)
+    base = blobs(rng, 500)
     dup = np.concatenate((base, base, base[:100]))[rng.permutation(1100)]
     for k in (2, 5, 24):
         ref = oracle.region_knn_pca(dup, k, want_knn=True)
@@ -143,7 +139,7 @@ def test_c1_size_cloud_k2000_sample_against_oracle(oracle):
     on the GPU, a slice of 600 queries checked against the brute-force oracle."""
     rg = pkg("region_growing")
     rng = np.random.default_rng(1)
-    pos = _blobs(rng, 200_000)
+    pos = blobs(rng, 200_000)
     torch.cuda.synchronize()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     dpos = torch.from_numpy(pos).cuda()
@@ -167,7 +163,7 @@ def test_floaters_do_not_degrade_the_grid(oracle):
     quantile range instead, so the search stays local -- and exact, outliers included."""
     rg = pkg("region_growing")
     rng = np.random.default_rng(8)
-    pos = _blobs(rng, 100_000)
+    pos = blobs(rng, 100_000)
     far = rng.uniform(-3000, 3000, size=(150, 3)).astype(np.float32)
     pos = np.concatenate((pos, far))[rng.permutation(100_150)]
     dpos = torch.from_numpy(pos).cuda()

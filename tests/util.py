@@ -32,6 +32,12 @@ LIFT_CASES = ["lift_bundled_halfres", "lift_lookat_fullres", "lift_lookat_rescal
 KMEANS_CASES = ["kmeans_color_k10", "kmeans_kdtree_k64_d59", "kmeans_converged_k4", "kmeans_empty_k8"]
 
 
+def blobs(rng, n, spread=0.3):
+    """float32 [n, 3]: ten Gaussian blobs of the given spread with centres in [-2, 2]^3."""
+    centres = rng.uniform(-2, 2, size=(10, 3))
+    return (centres[rng.integers(0, 10, n)] + rng.normal(0, spread, size=(n, 3))).astype(np.float32)
+
+
 def load_kmeans_case(name):
     z = np.load(os.path.join(GOLDEN, name + ".npz"))
     d = {k: z[k] for k in z.files}
