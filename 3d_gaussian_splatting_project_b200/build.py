@@ -18,8 +18,8 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "_obj")
 LIB = os.path.join(HERE, "libgslift.so")
-SOURCES = ["api.cu", "lift.cu", "lift_order.cu", "lift_sort.cu", "kmeans.cu", "kmeans_tc.cu", "kmeans_umma.cu",
-           "kmeans_ordered.cu", "ply_format.cu", "host_stage.cu", "viewer.cu", "region_growing.cu"]
+SOURCES = ["api.cu", "lift.cu", "lift_order.cu", "lift_sort.cu", "kmeans.cu", "kmeans_tc.cu", "kmeans_ordered.cu",
+           "ply_format.cu", "host_stage.cu", "viewer.cu", "region_growing.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

@@ -37,9 +37,6 @@ inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 // Cached per-device facts (SM count) so launches can size persistent grids.
 int sm_count();
 
-// lift.cu: one high-priority non-blocking helper stream per device, created on first use (NULL if that fails).
-cudaStream_t helper_stream();
-
 // kmeans_ordered.cu: scratch for gsl_kmeans_update_ordered.
 size_t ordered_workspace_bytes(int64_t N, int D, int K);
 
@@ -47,13 +44,5 @@ size_t ordered_workspace_bytes(int64_t N, int D, int K);
 bool tc_supported(int D, int K);
 int launch_step_tc(bool accumulate, const float *data, int64_t N, int D, const float *centroids, int K,
                    int32_t *labels, double *partials, int grid, cudaStream_t st);
-
-// kmeans_umma.cu: the same screening with tcgen05.mma / tensor memory, full 128-row tiles of a
-// 16-byte aligned matrix.  *rows_done = rows covered (0: not applicable), *n_parts = partial blocks written.
-bool umma_supported(int D, int K);
-int launch_step_umma(bool accumulate, const float *data, int64_t N, int D, const float *centroids, int K,
-                     int32_t *labels, double *partials, cudaStream_t st, int64_t *rows_done, int *n_parts);
-int launch_umma_selftest(const float *data, int64_t N, int D, const float *centroids, int K, int32_t *labels,
-                         unsigned long long *out2, cudaStream_t st, int64_t *rows_done);
 
 }  // namespace gsl

@@ -403,34 +403,11 @@ static bool allow_tc()
     return !(e && e[0] == '0');
 }
 
-// GSLIFT_KMEANS_UMMA=1 selects the tcgen05 screening kernel (kmeans_umma.cu) where it applies.  It
-// returns the same labels (tests run both) but is the slower of the two as measured in round 2
-// (1.77 - 1.99 ms per iteration at 6 M x 59, K = 64, against 1.19 ms for the mma.sync kernel with
-// two CTAs per SM: profiles/r2/ncu_kmeans_umma_*.txt), so it is opt-in.
-static bool allow_umma()
-{
-    const char *e = getenv("GSLIFT_KMEANS_UMMA");
-    return e && e[0] == '1';
-}
-
-// One assignment pass (+ per-CTA partial sums when kAcc).  *n_parts = partial blocks written.
+// One assignment pass (+ one block of partial sums per CTA when kAcc).
 template <bool kAcc>
 static int launch_step(const float *data, int64_t N, int D, const float *centroids, int K,
-                       int32_t *labels, double *partials, int grid, cudaStream_t st, int *n_parts)
+                       int32_t *labels, double *partials, int grid, cudaStream_t st)
 {
-    *n_parts = kAcc ? grid : 0;
-    if (!force_exact() && allow_tc() && allow_umma() && umma_supported(D, K)) {
-        int64_t done = 0;
-        int parts = 0;
-        if (int rc = launch_step_umma(kAcc, data, N, D, centroids, K, labels, partials, st, &done, &parts)) return rc;
-        if (done == N) { *n_parts = parts; return GSL_OK; }
-        if (done > 0) {
-            // rows past the last full tile: the mma.sync kernel, one CTA, its partial block right behind
-            *n_parts = kAcc ? parts + 1 : 0;
-            return launch_step_tc(kAcc, data + done * D, N - done, D, centroids, K, labels + done,
-                                  kAcc ? partials + (size_t)parts * K * (D + 1) : nullptr, 1, st);
-        }
-    }
     if (!force_exact() && allow_tc() && K >= 16 && tc_supported(D, K))
         return launch_step_tc(kAcc, data, N, D, centroids, K, labels, partials, grid, st);
     // the screened kernel pads the centroid block to DREG floats per row: fall back to the
@@ -456,8 +433,7 @@ extern "C" int gsl_kmeans_assign(const float *data, int64_t N, int D, const floa
     if (int rc = check_kd("gsl_kmeans_assign", N, D, K)) return rc;
     if (N == 0) return GSL_OK;
     if (!data || !centroids || !labels) return fail(GSL_EINVAL, "gsl_kmeans_assign: null pointer");
-    int unused = 0;
-    return launch_step<false>(data, N, D, centroids, K, labels, nullptr, step_grid(N), (cudaStream_t)stream, &unused);
+    return launch_step<false>(data, N, D, centroids, K, labels, nullptr, step_grid(N), (cudaStream_t)stream);
 }
 
 extern "C" int gsl_kmeans_step(const float *data, int64_t N, int D, const float *centroids, int K,
@@ -474,8 +450,8 @@ extern "C" int gsl_kmeans_step(const float *data, int64_t N, int D, const float 
     if (!data || !labels || !ws) return fail(GSL_EINVAL, "gsl_kmeans_step: null pointer");
     if (ws_bytes < gsl_kmeans_workspace_bytes(N, D, K)) return fail(GSL_EWORKSPACE, "gsl_kmeans_step: workspace %zu < %zu", ws_bytes, gsl_kmeans_workspace_bytes(N, D, K));
     double *partials = reinterpret_cast<double *>(((uintptr_t)ws + 255) & ~(uintptr_t)255);
-    int grid = step_grid(N);
-    if (int rc = launch_step<true>(data, N, D, centroids, K, labels, partials, grid, st, &grid)) return rc;
+    const int grid = step_grid(N);
+    if (int rc = launch_step<true>(data, N, D, centroids, K, labels, partials, grid, st)) return rc;
     kmeans_reduce_kernel<<<(n_el + 31) / 32, kReduceThreads, 0, st>>>(partials, grid, n_el, sums);
     GSL_LAUNCH_CHECK("kmeans_reduce_kernel");
     return GSL_OK;
@@ -509,7 +485,7 @@ extern "C" int gsl_kmeans_step_exchange(const float *data, int64_t N, int D, con
         if (ws_bytes < gsl_kmeans_workspace_bytes(N, D, K)) return fail(GSL_EWORKSPACE, "gsl_kmeans_step_exchange: workspace %zu < %zu", ws_bytes, gsl_kmeans_workspace_bytes(N, D, K));
         partials = reinterpret_cast<double *>(((uintptr_t)ws + 255) & ~(uintptr_t)255);
         grid = step_grid(N);
-        if (int rc = launch_step<true>(data, N, D, centroids, K, labels, partials, grid, st, &grid)) return rc;
+        if (int rc = launch_step<true>(data, N, D, centroids, K, labels, partials, grid, st)) return rc;
     }
     // how long a rank waits inside the kernel for its peers (milliseconds)
     const char *tmo = getenv("GSLIFT_EXCHANGE_TIMEOUT_MS");

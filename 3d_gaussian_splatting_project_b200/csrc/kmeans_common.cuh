@@ -148,98 +148,4 @@ __device__ __forceinline__ void accumulate_tile(double *__restrict__ acc, const 
     }
 }
 
-// The same sums, in the same order, straight from the member bits: warp w owns the clusters k = w (mod
-// n_warps) and, for each, walks the lane masks bits[k][0 .. n_warps) -- rows in ascending order -- adding
-// the rows lane-per-dimension in float64.  No cluster starts, no row order, hence two block barriers and
-// the warp-0-only scan fewer per tile than zero/bits/starts/order/accumulate.
-__device__ __forceinline__ void accumulate_from_bits(double *__restrict__ acc, const float *__restrict__ tile, int pitch,
-                                                     const unsigned *__restrict__ bits, int K, int D,
-                                                     int lane, int warp, int n_warps)
-{
-    for (int k = warp; k < K; k += n_warps) {
-        unsigned m[8];
-        int members = 0;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) {
-            m[w] = w < n_warps ? bits[k * n_warps + w] : 0u;
-            members += __popc(m[w]);
-        }
-        if (members == 0) continue;
-        for (int d0 = 0; d0 < D; d0 += 64) {
-            const int da = d0 + lane, db = da + 32;
-            const bool ina = da < D, inb = db < D;
-            double sa = 0.0, sb = 0.0;
-#pragma unroll
-            for (int w = 0; w < 8; ++w) {
-                unsigned mm = m[w];
-                while (mm) {                                 // warp-uniform: every lane holds the same mask
-                    const int r = w * 32 + __ffs(mm) - 1;
-                    mm &= mm - 1;
-                    const float *row = tile + r * pitch;
-                    if (ina) sa += (double)row[da];
-                    if (inb) sb += (double)row[db];
-                }
-            }
-            if (ina) acc[k * (D + 1) + da] += sa;
-            if (inb) acc[k * (D + 1) + db] += sb;
-        }
-        if (lane == 0) acc[k * (D + 1) + D] += (double)members;
-    }
-}
-
-// Per-cluster sums of one sorted tile, walking ROWS instead of clusters: with a few hundred rows and up to 64
-// clusters a cluster has a handful of members, so a loop per cluster is mostly overhead.  Warp w
-// takes the clusters whose first sorted row lies in [32 w, 32 w + 32): whole clusters, contiguous
-// sorted rows, about 32 of them, and no cluster is shared between warps -- the order of the float64
-// additions stays fixed.  Lane = dimension (and dimension + 32); the running sums of the current
-// cluster stay in registers and are added to the accumulator when the label changes.
-__device__ __forceinline__ void accumulate_rows(double *__restrict__ acc, const float *__restrict__ tile, int pitch,
-                                                const unsigned short *__restrict__ cstart,
-                                                const unsigned short *__restrict__ order, int K, int D,
-                                                int n_rows, int lane, int warp, int n_warps)
-{
-    const int per = (n_rows + n_warps - 1) / n_warps;
-    // first cluster of this warp / of the next warp: the first k with cstart[k] >= warp * per
-    auto first_cluster = [&](int row) {
-        if (row <= 0) return 0;
-        if (row >= n_rows) return K;
-        int best = K;
-        for (int k0 = 0; k0 < K; k0 += 32) {
-            const int k = k0 + lane;
-            const unsigned hit = __ballot_sync(0xffffffffu, k < K && (int)cstart[k] >= row);
-            if (hit) { best = k0 + __ffs(hit) - 1; break; }
-        }
-        return best;
-    };
-    const int ka = first_cluster(warp * per), kb = first_cluster((warp + 1) * per);
-    if (ka >= kb) return;
-    const int i0 = cstart[ka], i1 = cstart[kb];
-    const int da = lane, db = lane + 32;
-    const bool ina = da < D, inb = db < D;
-    int k = ka, k_end = cstart[ka + 1];
-    double sa = 0.0, sb = 0.0;
-    int members = 0;
-    for (int i = i0; i < i1; ++i) {
-        while (i >= k_end) {                              // label changes: flush the finished cluster (warp-uniform)
-            if (members) {
-                if (ina) acc[k * (D + 1) + da] += sa;
-                if (inb) acc[k * (D + 1) + db] += sb;
-                if (lane == 0) acc[k * (D + 1) + D] += (double)members;
-                sa = 0.0; sb = 0.0; members = 0;
-            }
-            ++k;
-            k_end = cstart[k + 1];
-        }
-        const float *row = tile + (int)order[i] * pitch;
-        if (ina) sa += (double)row[da];
-        if (inb) sb += (double)row[db];
-        ++members;
-    }
-    if (members) {
-        if (ina) acc[k * (D + 1) + da] += sa;
-        if (inb) acc[k * (D + 1) + db] += sb;
-        if (lane == 0) acc[k * (D + 1) + D] += (double)members;
-    }
-}
-
 }  // namespace gsl

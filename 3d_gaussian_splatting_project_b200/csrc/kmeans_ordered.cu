@@ -13,18 +13,13 @@
 //                            (warp match_any ranks keep ascending row order)
 //   ordered_gather_kernel    member rows in list order into a contiguous, padded array per 32-dim chunk
 //   ordered_stream_kernel    one warp per (cluster, 32 dims): TMA bulk copies of its contiguous rows into
-//                            a shared-memory ring, added in order, lane = dimension (the default)
-//   ordered_chain_kernel     the round-1 form (GSLIFT_ORDERED_STREAM=0): CTA per (cluster, 32 dims), seven
-//                            producer warps cp.async member rows into a 4-deep shared-memory ring while
-//                            warp 0 adds them in order.  (Round 2 also tried one CTA per cluster with an
-//                            mbarrier-advanced ring fed by per-row cp.async: 12.5 ms against 4.5 ms.)
+//                            a shared-memory ring, added in order, lane = dimension
 //   shift_kernel             ||new - old||_F
 //
 // This is the parity mode (single device).  The throughput mode is gsl_kmeans_step's float64
 // segmented reduction, which is sharded and all-reduced.
-#include <stdlib.h>
-
 #include <algorithm>
+#include <mutex>
 
 #include "common.cuh"
 #include "kmeans_screen.cuh"
@@ -137,125 +132,18 @@ ordered_scatter_kernel(const int32_t *__restrict__ labels, int64_t N, int K,
     }
 }
 
-// grid (K, ceil(D/32)); lane = dimension d0 + lane.  Warp 0 is the consumer: it owns the K*D/32
-// float32 accumulators of this (cluster, dimension chunk) and adds member rows strictly in index
-// order.  Warps 1..7 are producers: they gather the member rows (128 bytes per row and chunk) with
-// cp.async straight into a ring of kChainRing shared-memory batches, three batches ahead of the
-// consumer, so the DRAM latency of the row gather is hidden behind the dependent add chain.
-constexpr int kChainRows = 7 * 32;     // rows per batch: 32 per producer warp
-constexpr int kChainRing = 4;
-
-__device__ __forceinline__ void cp_async_4(float *dst, const float *src)
-{
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((uint32_t)__cvta_generic_to_shared(dst)), "l"(src) : "memory");
-}
-
-__global__ void __launch_bounds__(kOrdThreads)
-ordered_chain_kernel(const float *__restrict__ data, int D, const int32_t *__restrict__ members,
-                     const int64_t *__restrict__ start, const int64_t *__restrict__ total,
-                     const float *__restrict__ old_c, float *__restrict__ new_c)
-{
-    extern __shared__ float buf[];              // [kChainRing][kChainRows][32]
-    const int k = blockIdx.x, d = blockIdx.y * 32 + (threadIdx.x & 31);
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int64_t n = total[k], s0 = start[k];
-    const bool live = d < D;
-    if (n == 0) {
-        if (w == 0 && live) new_c[(size_t)k * D + d] = old_c[(size_t)k * D + d];   // km:126 else-branch
-        return;
-    }
-    const int64_t n_batches = (n + kChainRows - 1) / kChainRows;
-    // producers: this warp's 32 rows of batch b.  The member indices of a batch are loaded one
-    // iteration before its copies are issued (load_idx -> issue): otherwise the latency of that
-    // load (~1 us) sits in front of every batch's cp.async and, through the barrier, in front of the
-    // consumer (profiles/r1/ncu_ordered_chain_r1.txt: the producers' first SHFL held 20 % of all samples).
-    auto load_idx = [&](int64_t b) -> int {
-        if (w > 0 && b < n_batches) {
-            const int64_t mi = b * kChainRows + (w - 1) * 32 + lane;
-            return mi < n ? __ldg(members + s0 + mi) : -1;
-        }
-        return -1;
-    };
-    // per row: one broadcast shared load (the row index, parked there by the lane that fetched it),
-    // one 32 x 32 -> 64-bit multiply-add (the source address) and the copy itself -- the seven
-    // producer warps share the SM's issue slots with the consumer.  (Broadcasting the indices with
-    // shuffles compiled to a dozen instructions per row: the warp-uniform branch around them is not
-    // provably convergent, so every shuffle came with its own collective-sync scaffolding.)
-    __shared__ int idx_s[7 * 32];
-    const char *base = reinterpret_cast<const char *>(data + (live ? d : 0));
-    asm volatile("" : "+l"(base));                               // keep it in registers, do not re-derive it per row
-    const unsigned row_bytes = (unsigned)D * 4u;
-    const unsigned buf_s = (unsigned)__cvta_generic_to_shared(buf);
-    auto issue = [&](int64_t b, int idx) {
-        if (w > 0 && b < n_batches) {
-            int *mine = idx_s + (w - 1) * 32;
-            __syncwarp();                                        // the previous batch's reads of this warp's slots are done
-            mine[lane] = idx;
-            __syncwarp();
-            unsigned dst = buf_s + (((unsigned)(b % kChainRing) * kChainRows + (unsigned)(w - 1) * 32u) * 32u + (unsigned)lane) * 4u;
-            asm volatile("" : "+r"(dst));                        // one register plus an immediate per row
-#pragma unroll
-            for (int j0 = 0; j0 < 32; j0 += 8) {
-                int r[8];
-#pragma unroll
-                for (int j = 0; j < 8; ++j) r[j] = mine[j0 + j];
-#pragma unroll
-                for (int j = 0; j < 8; ++j)
-                    if (live && r[j] >= 0)
-                        asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst + (unsigned)(j0 + j) * 128u), "l"(base + (size_t)(unsigned)r[j] * row_bytes) : "memory");
-            }
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-    };
-    for (int p = 0; p < kChainRing - 1; ++p) issue(p, load_idx(p));
-    int idx_next = load_idx(kChainRing - 1);
-    float acc = -0.0f;              // (-0) + x == x for every x: same as starting from the first row
-    for (int64_t b = 0; b < n_batches; ++b) {
-        asm volatile("cp.async.wait_group %0;" ::"n"(kChainRing - 2) : "memory");   // my part of batch b landed
-        __syncthreads();            // everyone's part landed; the consumer is done with batch b - 1
-        issue(b + kChainRing - 1, idx_next);    // refills the slot batch b - 1 occupied
-        idx_next = load_idx(b + kChainRing);    // in flight while the consumer adds batch b
-        if (w == 0 && live) {
-            const int cnt = (int)min((int64_t)kChainRows, n - b * kChainRows);
-            const float *src = buf + (size_t)(b % kChainRing) * kChainRows * 32 + lane;
-            // the adds are one dependent chain (4 cycles each); the shared loads of the NEXT 32
-            // values are issued before the 32 adds of the current ones, so the chain does not wait
-            // for shared memory inside a batch
-            int i = 0;
-            if (cnt >= 32) {
-                float x[32], y[32];
-#pragma unroll
-                for (int j = 0; j < 32; ++j) x[j] = src[j * 32];
-                for (; i + 64 <= cnt; i += 32) {
-#pragma unroll
-                    for (int j = 0; j < 32; ++j) y[j] = src[(i + 32 + j) * 32];
-#pragma unroll
-                    for (int j = 0; j < 32; ++j) acc = __fadd_rn(acc, x[j]);
-#pragma unroll
-                    for (int j = 0; j < 32; ++j) x[j] = y[j];
-                }
-#pragma unroll
-                for (int j = 0; j < 32; ++j) acc = __fadd_rn(acc, x[j]);
-                i += 32;
-            }
-            for (; i < cnt; ++i) acc = __fadd_rn(acc, src[i * 32]);
-        }
-    }
-    if (w == 0 && live) new_c[(size_t)k * D + d] = (float)((double)acc / (double)n);
-}
-
-// ---- streamed form of the chain (default) --------------------------------------------------------
-// The chain kernel above has to collect its member rows with one 4-byte cp.async per lane and row
-// (rows of D = 59 floats are only 4-byte aligned), and ncu shows that this is what paces it: 224
-// such instructions per batch and SM, ~2750 cycles per batch against ~900 for the 224 dependent
-// adds.  Splitting the work removes the gather from the serial part:
+// ---- the chains: gather, then stream ---------------------------------------------------------------
+// A chain that collects its own member rows needs one 4-byte copy per lane and row (rows of D = 59
+// floats are only 4-byte aligned), and that, not the dependent adds, is what paces it: measured
+// ~2750 cycles per 224-row batch against ~900 for the 224 adds.  Splitting the work removes the
+// gather from the serial part:
 //   ordered_gather_kernel   fully parallel and bandwidth bound: member rows in list order into a
 //                           contiguous array per 32-dimension chunk (128 bytes per row and chunk,
 //                           zero padded; layout below)
 //   ordered_stream_kernel   one WARP per (cluster, chunk): its rows are one contiguous, 16-byte
-//                           aligned stream, fetched by TMA bulk copies of 256 rows (one instruction
-//                           per 32 KB, completion on an mbarrier) four stages ahead, and added in
-//                           order, lane = dimension.  No other warp, no block barrier.
+//                           aligned stream, fetched by TMA bulk copies of up to 512 rows (one
+//                           instruction per 64 KB stage, completion on an mbarrier) two stages ahead,
+//                           and added in order, lane = dimension.  No other warp, no block barrier.
 constexpr int kStreamRows = 512;       // rows per stage (64 KB)
 constexpr int kStreamStages = 3;
 
@@ -415,7 +303,7 @@ static OrdWs ordered_layout(int64_t N, int D, int K)
     o.start = off;       off += align_up((size_t)K * sizeof(int64_t), 256);
     o.pstart = off;      off += align_up((size_t)(K + 1) * sizeof(int64_t), 256);
     o.members = off;     off += align_up((size_t)N * sizeof(int32_t), 256);
-    // streamed form: the member rows per 32-dimension chunk, 128 bytes each (the TMA copies want 16-byte
+    // the member rows per 32-dimension chunk, 128 bytes each (the TMA copies want 16-byte
     // aligned sources; the slot count is padded so that every chunk starts on a 256-byte boundary)
     o.slots_pad = align_up((size_t)(N > 0 ? N : 1) + 4 * (size_t)K, 4);      // every cluster padded to whole groups of four
     o.rows32 = off;      off += align_up((size_t)((D + 31) / 32) * o.slots_pad * 32 * sizeof(float), 256);
@@ -424,6 +312,27 @@ static OrdWs ordered_layout(int64_t N, int D, int K)
 }
 
 size_t ordered_workspace_bytes(int64_t N, int D, int K) { return ordered_layout(N, D, K).bytes; }
+
+// The stream on which gsl_kmeans_update_ordered runs the chains of the big clusters while the
+// caller's stream gathers and sums the others (see in_phase).  High priority and non-blocking; one
+// per device, created on first use (NULL if that fails).
+static cudaStream_t helper_stream()
+{
+    static std::mutex mu;
+    static cudaStream_t streams[64] = {};
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
+    std::lock_guard<std::mutex> lock(mu);
+    if (!streams[dev]) {
+        int lo = 0, hi = 0;
+        cudaDeviceGetStreamPriorityRange(&lo, &hi);
+        if (cudaStreamCreateWithPriority(&streams[dev], cudaStreamNonBlocking, hi) != cudaSuccess) {
+            cudaGetLastError();
+            streams[dev] = nullptr;
+        }
+    }
+    return streams[dev];
+}
 
 }  // namespace gsl
 
@@ -466,47 +375,39 @@ extern "C" int gsl_kmeans_update_ordered(const float *data, const int32_t *label
         ordered_scatter_kernel<<<n_tiles, kOrdThreads, sc_smem, st>>>(labels, N, K, tile_counts, start, members);
         GSL_LAUNCH_CHECK("ordered_scatter_kernel");
     }
-    dim3 grid((unsigned)K, (unsigned)((D + 31) / 32));
-    static const bool streamed = [] { const char *e = getenv("GSLIFT_ORDERED_STREAM"); return !(e && e[0] == '0'); }();
-    if (streamed) {
-        float *rows32 = reinterpret_cast<float *>(base + L.rows32 - 256);
-        const size_t st_smem = (size_t)kStreamStages * kStreamRows * 32 * sizeof(float);
-        GSL_CUDA_TRY(cudaFuncSetAttribute(ordered_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)st_smem));
-        const int64_t warps = (N + 3) / 4 + K;
-        const unsigned g = (unsigned)std::min<int64_t>((warps * 32 + 255) / 256, (int64_t)sm_count() * 16);
-        auto gather = [&](int phase, cudaStream_t s) -> int {
-            if (N == 0) return GSL_OK;
-            ordered_gather_kernel<<<g, 256, 0, s>>>(data, D, (int)grid.y, members, start, pstart, total, K, (int64_t)L.slots_pad, rows32, phase);
-            GSL_LAUNCH_CHECK("ordered_gather_kernel");
-            return GSL_OK;
-        };
-        auto chains = [&](int phase, cudaStream_t s) -> int {
-            ordered_stream_kernel<<<grid, 32, st_smem, s>>>(rows32, (int64_t)L.slots_pad, D, K, start, pstart, total, old_centroids, new_centroids, phase);
-            GSL_LAUNCH_CHECK("ordered_stream_kernel");
-            return GSL_OK;
-        };
-        cudaStream_t side = N >= (1 << 18) ? helper_stream() : nullptr;
-        cudaEvent_t ev = nullptr;
-        if (side && cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); side = nullptr; }
-        if (!side) {
-            if (int rc = gather(0, st)) return rc;
-            if (int rc = chains(0, st)) return rc;
-        } else {
-            int rc = gather(1, st);
-            if (rc == GSL_OK && (cudaEventRecord(ev, st) != cudaSuccess || cudaStreamWaitEvent(side, ev, 0) != cudaSuccess)) rc = fail(GSL_ECUDA, "gsl_kmeans_update_ordered: fork failed");
-            if (rc == GSL_OK) rc = chains(1, side);
-            if (rc == GSL_OK) rc = gather(2, st);
-            if (rc == GSL_OK) rc = chains(2, st);
-            // the caller's stream continues only after the big clusters' chains (also when something above failed)
-            if (cudaEventRecord(ev, side) != cudaSuccess || cudaStreamWaitEvent(st, ev, 0) != cudaSuccess) { if (rc == GSL_OK) rc = fail(GSL_ECUDA, "gsl_kmeans_update_ordered: join failed"); }
-            cudaEventDestroy(ev);
-            if (rc != GSL_OK) return rc;
-        }
+    const dim3 grid((unsigned)K, (unsigned)((D + 31) / 32));
+    float *rows32 = reinterpret_cast<float *>(base + L.rows32 - 256);
+    const size_t st_smem = (size_t)kStreamStages * kStreamRows * 32 * sizeof(float);
+    GSL_CUDA_TRY(cudaFuncSetAttribute(ordered_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)st_smem));
+    const int64_t warps = (N + 3) / 4 + K;
+    const unsigned g = (unsigned)std::min<int64_t>((warps * 32 + 255) / 256, (int64_t)sm_count() * 16);
+    auto gather = [&](int phase, cudaStream_t s) -> int {
+        if (N == 0) return GSL_OK;
+        ordered_gather_kernel<<<g, 256, 0, s>>>(data, D, (int)grid.y, members, start, pstart, total, K, (int64_t)L.slots_pad, rows32, phase);
+        GSL_LAUNCH_CHECK("ordered_gather_kernel");
+        return GSL_OK;
+    };
+    auto chains = [&](int phase, cudaStream_t s) -> int {
+        ordered_stream_kernel<<<grid, 32, st_smem, s>>>(rows32, (int64_t)L.slots_pad, D, K, start, pstart, total, old_centroids, new_centroids, phase);
+        GSL_LAUNCH_CHECK("ordered_stream_kernel");
+        return GSL_OK;
+    };
+    cudaStream_t side = N >= (1 << 18) ? helper_stream() : nullptr;
+    cudaEvent_t ev = nullptr;
+    if (side && cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); side = nullptr; }
+    if (!side) {
+        if (int rc = gather(0, st)) return rc;
+        if (int rc = chains(0, st)) return rc;
     } else {
-        const size_t ch_smem = (size_t)kChainRing * kChainRows * 32 * sizeof(float);
-        GSL_CUDA_TRY(cudaFuncSetAttribute(ordered_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ch_smem));
-        ordered_chain_kernel<<<grid, kOrdThreads, ch_smem, st>>>(data, D, members, start, total, old_centroids, new_centroids);
-        GSL_LAUNCH_CHECK("ordered_chain_kernel");
+        int rc = gather(1, st);
+        if (rc == GSL_OK && (cudaEventRecord(ev, st) != cudaSuccess || cudaStreamWaitEvent(side, ev, 0) != cudaSuccess)) rc = fail(GSL_ECUDA, "gsl_kmeans_update_ordered: fork failed");
+        if (rc == GSL_OK) rc = chains(1, side);
+        if (rc == GSL_OK) rc = gather(2, st);
+        if (rc == GSL_OK) rc = chains(2, st);
+        // the caller's stream continues only after the big clusters' chains (also when something above failed)
+        if (cudaEventRecord(ev, side) != cudaSuccess || cudaStreamWaitEvent(st, ev, 0) != cudaSuccess) { if (rc == GSL_OK) rc = fail(GSL_ECUDA, "gsl_kmeans_update_ordered: join failed"); }
+        cudaEventDestroy(ev);
+        if (rc != GSL_OK) return rc;
     }
     shift_kernel<<<1, 256, 0, st>>>(new_centroids, old_centroids, K * D, shift, bad_label);
     GSL_LAUNCH_CHECK("shift_kernel");

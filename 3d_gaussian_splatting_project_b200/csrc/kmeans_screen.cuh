@@ -1,6 +1,6 @@
-// Device helpers shared by the two screened K-means assignment kernels (kmeans_tc.cu: mma.sync,
-// kmeans_umma.cu: tcgen05): TF32 rounding, the TMA bulk copy of a row tile, the screening bound and
-// the float32 / float64 refinement of the candidates (stages B and C, see kmeans_tc.cu).
+// Device helpers of the tensor-core screened K-means assignment kernel (kmeans_tc.cu): TF32
+// rounding, the TMA bulk copy of a row tile, the screening bound and the float32 / float64
+// refinement of the candidates (stages B and C, see kmeans_tc.cu).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>

@@ -23,8 +23,6 @@
 //
 // The per-cluster float64 sums that follow are the shared segmented reduction
 // (kmeans_common.cuh).  Compiled with -fmad=false.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "kmeans_common.cuh"
 #include "kmeans_screen.cuh"
@@ -133,7 +131,7 @@ template <bool kAccumulate, bool kCheck>
 __global__ void __launch_bounds__(kTcThreads, 2)
 kmeans_step_tc_kernel(const float *__restrict__ data, int64_t N, int D, const float *__restrict__ centroids,
                       int K, int32_t *__restrict__ labels, double *__restrict__ partials,
-                      TcSmem L, int vec_ok, float eps, unsigned long long *__restrict__ check_out, int row_walk)
+                      TcSmem L, int vec_ok, float eps, unsigned long long *__restrict__ check_out)
 {
     extern __shared__ __align__(16) unsigned char smem[];
     double *acc = reinterpret_cast<double *>(smem + L.acc);
@@ -281,18 +279,11 @@ kmeans_step_tc_kernel(const float *__restrict__ data, int64_t N, int D, const fl
         if (kAccumulate) {
             const unsigned same = tile_member_bits(bits, mine, kTcThreads / 32, lane, warp);
             __syncthreads();
-            if (row_walk == 3) {
-                // experiment: sums straight from the member bits, no sort (same order of additions; two barriers
-                // fewer, but measured slower: 1.30 vs 1.15 ms per step -- the mask walk is a serial, branchy chain)
-                accumulate_from_bits(acc, tile, pitch, bits, K, D, lane, warp, kTcThreads / 32);
-            } else {
-                if (warp == 0) tile_cluster_starts(bits, cstart, K, kTcThreads / 32, lane);
-                __syncthreads();
-                tile_row_order(bits, cstart, order, mine, same, kTcThreads / 32, t, lane, warp);
-                __syncthreads();
-                if (row_walk == 1) accumulate_rows(acc, tile, pitch, cstart, order, K, D, kTcRows, lane, warp, kTcThreads / 32);
-                else accumulate_tile(acc, tile, pitch, cstart, order, K, D, lane, warp, kTcThreads / 32);
-            }
+            if (warp == 0) tile_cluster_starts(bits, cstart, K, kTcThreads / 32, lane);
+            __syncthreads();
+            tile_row_order(bits, cstart, order, mine, same, kTcThreads / 32, t, lane, warp);
+            __syncthreads();
+            accumulate_tile(acc, tile, pitch, cstart, order, K, D, lane, warp, kTcThreads / 32);
         }
         __syncthreads();                                 // every reader of the tile is done
         const int64_t nxt = tl + gridDim.x;
@@ -324,10 +315,7 @@ static int launch_tc_t(const float *data, int64_t N, int D, const float *centroi
     GSL_CUDA_TRY(cudaFuncSetAttribute(kmeans_step_tc_kernel<kAcc, kCheck>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total));
     const int vec_ok = (((uintptr_t)data & 15) == 0);        // 256 rows x D floats is always a multiple of 16 bytes
     const float eps = (float)((D + 12) * 5.9604644775390625e-08);
-    // experiments: GSLIFT_KMEANS_ROWWALK = 1: walk the sorted rows; 3: no sort, clusters walk their member bits;
-    // default 0: sort the tile's rows by label, clusters walk their rows
-    const char *rw = getenv("GSLIFT_KMEANS_ROWWALK");
-    kmeans_step_tc_kernel<kAcc, kCheck><<<grid, kTcThreads, L.total, st>>>(data, N, D, centroids, K, labels, partials, L, vec_ok, eps, check_out, rw ? atoi(rw) : 0);
+    kmeans_step_tc_kernel<kAcc, kCheck><<<grid, kTcThreads, L.total, st>>>(data, N, D, centroids, K, labels, partials, L, vec_ok, eps, check_out);
     GSL_LAUNCH_CHECK("kmeans_step_tc_kernel");
     return GSL_OK;
 }
@@ -349,13 +337,6 @@ extern "C" int gsl_kmeans_screen_selftest(const float *data, int64_t N, int D, c
     if (!data || !centroids || !labels || !out2 || N < 0) return fail(GSL_EINVAL, "gsl_kmeans_screen_selftest: bad argument");
     if (!tc_supported(D, K)) return fail(GSL_EINVAL, "gsl_kmeans_screen_selftest: needs K <= 64 and 8 <= D <= 64");
     if (N == 0) return GSL_OK;
-    // with GSLIFT_KMEANS_UMMA=1: full 128-row tiles through the tcgen05 kernel, the rest through mma.sync
-    int64_t done = 0;
-    const char *e = getenv("GSLIFT_KMEANS_UMMA");
-    if (e && e[0] == '1')
-        if (int rc = launch_umma_selftest(data, N, D, centroids, K, labels, out2, (cudaStream_t)stream, &done)) return rc;
-    if (done == N) return GSL_OK;
-    data += done * D; labels += done; N -= done;
     const int64_t tiles = (N + kTcRows - 1) / kTcRows;
     const int64_t cap = (int64_t)sm_count() * 2;
     return launch_tc_t<false, true>(data, N, D, centroids, K, labels, nullptr, (int)(tiles < cap ? tiles : cap), out2, (cudaStream_t)stream);

@@ -2,8 +2,6 @@
 // cell.  The sort is a preprocessing utility, not part of the vote arithmetic, and uses CUB's
 // device radix sort (three 8-bit passes) from the CUDA toolkit; its scratch comes out of the
 // caller's workspace like everything else.
-#include <stdlib.h>
-
 #include <cub/device/device_radix_sort.cuh>
 
 #include "common.cuh"
@@ -27,9 +25,8 @@ int sort_cells(const uint32_t *keys_in, uint32_t *keys_out, const int32_t *idx_i
     // The order only has to make tiles compact, it need not be total.  Up to 2 M Gaussians a 65536-cell grid
     // (the top 16 key bits, two 8-bit passes) already holds ~30 per cell, and the third pass costs more than the
     // slightly looser tiles (measured at 750 K: pass 0.576 -> 0.560 ms; at 6 M the gather loses what the sort
-    // gains, so the full 24-bit order stays).  GSLIFT_SORT_LOW_BIT overrides (experiments).
-    static const int forced = [] { const char *e = getenv("GSLIFT_SORT_LOW_BIT"); const int v = e ? atoi(e) : -1; return v > 16 ? 16 : v; }();
-    const int low = forced >= 0 ? forced : (N <= (2 << 20) ? 8 : 0);
+    // gains, so the full 24-bit order stays).
+    const int low = N <= (2 << 20) ? 8 : 0;
     GSL_CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, need, keys_in, keys_out, idx_in, idx_out, (int)N, low, 24, st));
     if (need > temp_bytes) return fail(GSL_EWORKSPACE, "ordering: sort scratch %zu > reserved %zu", need, temp_bytes);
     GSL_CUDA_TRY(cub::DeviceRadixSort::SortPairs(temp, need, keys_in, keys_out, idx_in, idx_out, (int)N, low, 24, st));

@@ -131,14 +131,6 @@ def test_screened_assignment_equals_float64_scan(oracle, monkeypatch):
         monkeypatch.delenv("GSLIFT_KMEANS_EXACT", raising=False)
         assert np.array_equal(fast, slow), f"{name}: screening changed {(fast != slow).sum()} labels"
         assert np.array_equal(fast, fast2), name
-        # the tcgen05 (UMMA / tensor memory) screening kernel is opt-in; same labels, same sums
-        monkeypatch.setenv("GSLIFT_KMEANS_UMMA", "1")
-        umma_lab, umma_sums = ops.kmeans_step(dev(data), dev(cen))
-        monkeypatch.delenv("GSLIFT_KMEANS_UMMA")
-        assert np.array_equal(umma_lab.cpu().numpy(), fast), f"{name}: tcgen05 and mma.sync screening disagree on {(umma_lab.cpu().numpy() != fast).sum()} rows"
-        if np.isfinite(data).all() and np.abs(data).max() < 1e18:
-            ref_sums = ops.kmeans_step(dev(data), dev(cen))[1]
-            assert torch.equal(umma_sums[:, -1], ref_sums[:, -1]) and torch.allclose(umma_sums, ref_sums, rtol=1e-12, atol=1e-300), name
         assert np.array_equal(fast.astype(np.int64), want), f"{name}: {(fast != want).sum()} differ from the oracle (ties {int((gap == 0).sum())})"
 
 
@@ -158,23 +150,16 @@ def test_tensor_core_screening_bound_holds_on_data():
     sets.append(("far offset, tight", off, off[rng.choice(len(off), 40, replace=False)]))
     wide = (rng.standard_normal((100_000, 8)) * np.array([1e-3, 1, 1e3, 1, 1, 1e2, 1, 1e-2])).astype(np.float32)
     sets.append(("mixed scales D=8", wide, wide[rng.choice(len(wide), 16, replace=False)]))
-    import os
     for name, x, c in sets:
-        for kernel in ("mma.sync", "tcgen05"):          # both tensor-core screening kernels rely on the same bound
-            if kernel == "tcgen05":
-                os.environ["GSLIFT_KMEANS_UMMA"] = "1"
-            try:
-                out = torch.zeros(2, dtype=torch.int64, device=DEV)
-                labels = torch.empty(len(x), dtype=torch.int32, device=DEV)
-                dx, dc = dev(x), dev(c)
-                native.check(native.lib().gsl_kmeans_screen_selftest(dx.data_ptr(), len(x), x.shape[1], dc.data_ptr(), len(c),
-                                                                     labels.data_ptr(), out.data_ptr(), None))
-                torch.cuda.synchronize()
-            finally:
-                os.environ.pop("GSLIFT_KMEANS_UMMA", None)
-            viol, cand = (int(v) for v in out.tolist())
-            print(f"[tc screen, {kernel}] {name}: bound violations {viol}, candidates per row {cand / len(x):.3f}")
-            assert viol == 0
+        out = torch.zeros(2, dtype=torch.int64, device=DEV)
+        labels = torch.empty(len(x), dtype=torch.int32, device=DEV)
+        dx, dc = dev(x), dev(c)
+        native.check(native.lib().gsl_kmeans_screen_selftest(dx.data_ptr(), len(x), x.shape[1], dc.data_ptr(), len(c),
+                                                             labels.data_ptr(), out.data_ptr(), None))
+        torch.cuda.synchronize()
+        viol, cand = (int(v) for v in out.tolist())
+        print(f"[tc screen] {name}: bound violations {viol}, candidates per row {cand / len(x):.3f}")
+        assert viol == 0
 
 
 def test_ties_duplicates_and_determinism(oracle):
