@@ -1,10 +1,12 @@
 // Reference-order centroid update for sm_100a.
 //
 // NumPy evaluates `data[labels == c].mean(axis=0)` (3D_clustering/k_means.py:125-128) as a
-// float32 SEQUENTIAL sum over the members in index order, then one float64 division rounded
-// to float32 (see oracle/gsl_oracle.c: orc_kmeans_update).  Float32 addition is not
-// associative, so reproducing the reference bit for bit means keeping that order: one serial
-// chain per (cluster, dimension).  The K*D chains are independent, so the work is:
+// float32 sum started from the identity +0.0, then one float64 division rounded to float32 (see
+// oracle/gsl_oracle.c: orc_kmeans_update).  For D >= 2 the sum is SEQUENTIAL over the members in
+// index order; for D = 1 the reduced axis is contiguous and NumPy uses its pairwise summation
+// (ordered_pairwise_kernel below).  Float32 addition is not associative, so reproducing the
+// reference bit for bit means keeping that order: one serial chain per (cluster, dimension).
+// The K*D chains are independent, so the work is:
 //
 //   ordered_count_kernel     per 1024-row tile, member count per cluster
 //   ordered_scan_kernel      per cluster, exclusive scan of the tile counts (+ totals)
@@ -14,6 +16,8 @@
 //   ordered_gather_kernel    member rows in list order into a contiguous, padded array per 32-dim chunk
 //   ordered_stream_kernel    one warp per (cluster, 32 dims): TMA bulk copies of its contiguous rows into
 //                            a shared-memory ring, added in order, lane = dimension
+//   (D = 1: ordered_column_kernel gathers the members into one dense column and
+//    ordered_pairwise_kernel sums each cluster's slice of it with NumPy's pairwise tree)
 //   shift_kernel             ||new - old||_F
 //
 // This is the parity mode (single device).  The throughput mode is gsl_kmeans_step's float64
@@ -75,10 +79,21 @@ ordered_scan_kernel(int32_t *__restrict__ tile_counts, int n_tiles, int K, int64
     }
 }
 
+// The chain of the largest cluster is the critical path (2.2 ms at C5, where one cluster holds 12 % of the
+// rows), the gather in front of it is not: clusters with at least 1/16 of the (valid) members are gathered
+// first and their chains start on a helper stream while the caller's stream gathers and sums the rest.
+//   phase 0: every cluster   1: the big ones   2: the others
+__device__ __forceinline__ bool in_phase(int phase, int64_t n, int64_t n_members)
+{
+    const bool big = n * 16 >= n_members && n > 0;
+    return phase == 0 || (phase == 1) == big;
+}
+
 // start[k] = members before cluster k; pstart[k] = the same with every cluster padded to a multiple of four
-// rows (pstart[K] = padded total): the streamed chain reads its rows in groups of four.
+// rows (pstart[K] = padded total): the streamed chain reads its rows in groups of four.  *n_big = the number
+// of clusters that phase 1 takes (second word of the workspace header, read by the tests).
 __global__ void ordered_start_kernel(const int64_t *__restrict__ total, int K, int64_t *__restrict__ start,
-                                     int64_t *__restrict__ pstart)
+                                     int64_t *__restrict__ pstart, int *__restrict__ n_big)
 {
     if (threadIdx.x == 0 && blockIdx.x == 0) {
         int64_t run = 0, prun = 0;
@@ -89,6 +104,9 @@ __global__ void ordered_start_kernel(const int64_t *__restrict__ total, int K, i
             prun += (total[k] + 3) & ~(int64_t)3;
         }
         pstart[K] = prun;
+        int big = 0;
+        for (int k = 0; k < K; ++k) big += in_phase(1, total[k], run);
+        *n_big = big;
     }
 }
 
@@ -146,16 +164,6 @@ ordered_scatter_kernel(const int32_t *__restrict__ labels, int64_t N, int K,
 //                           and added in order, lane = dimension.  No other warp, no block barrier.
 constexpr int kStreamRows = 512;       // rows per stage (64 KB)
 constexpr int kStreamStages = 3;
-
-// The chain of the largest cluster is the critical path (2.2 ms at C5, where one cluster holds 12 % of the
-// rows), the gather in front of it is not: clusters with at least 1/16 of the members are gathered first and
-// their chains start on a helper stream while the caller's stream gathers and sums the rest.
-//   phase 0: every cluster   1: the big ones   2: the others
-__device__ __forceinline__ bool in_phase(int phase, int64_t n, int64_t n_members)
-{
-    const bool big = n * 16 >= n_members && n > 0;
-    return phase == 0 || (phase == 1) == big;
-}
 
 // rows32[chunk][group][lane][4]: the rows of a cluster start at a multiple of four slots (pstart), four
 // consecutive rows form a group, and a lane's four values of a group are contiguous -- the stream kernel
@@ -223,7 +231,7 @@ ordered_stream_kernel(const float *__restrict__ rows32, int64_t slots_pad, int D
         }
     };
     for (int b = 0; b < kStreamStages - 1; ++b) issue(b);
-    float acc = -0.0f;              // (-0) + x == x for every x: same as starting from the first row
+    float acc = 0.0f;               // NumPy's add.reduce starts from its identity: a column of -0.0 sums to +0.0
     for (int64_t b = 0; b < n_batches; ++b) {
         __syncwarp();               // every lane is done reading batch b - 1, whose stage is refilled now
         issue(b + kStreamStages - 1);
@@ -271,6 +279,118 @@ ordered_stream_kernel(const float *__restrict__ rows32, int64_t slots_pad, int D
     if (live) new_c[(size_t)k * D + d] = (float)((double)acc / (double)n);
 }
 
+// ---- D = 1: NumPy's pairwise sum ---------------------------------------------------------------------
+// With one feature, data[mask] is an (n, 1) array whose reduced axis is contiguous, and NumPy's add loop
+// sums it with pairwise_sum (numpy/_core/src/umath/loops_utils.h.src), float32 throughout:
+//   n < 8          plain adds
+//   n <= 128       eight strided accumulators, ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)), then the tail in order
+//   n > 128        split at n2 = n/2 - (n/2 mod 8): pairwise(first n2) + pairwise(the rest)
+// One tree over the whole member list.  Its shape depends on n only, so subtrees can be summed apart and
+// combined in the tree's order.
+constexpr int kPwBlock = 128;          // NumPy's PW_BLOCKSIZE
+constexpr int kPwLevels = 10;          // top levels of the tree spread over the threads of one block
+constexpr int kPwThreads = 1 << kPwLevels;
+
+__device__ __forceinline__ int64_t pairwise_split(int64_t n)
+{
+    const int64_t h = n / 2;
+    return h - h % 8;
+}
+
+__device__ float pairwise_leaf(const float *a, int n)      // n <= kPwBlock
+{
+    if (n < 8) {
+        float r = 0.0f;
+        for (int i = 0; i < n; ++i) r = __fadd_rn(r, a[i]);
+        return r;
+    }
+    float r[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) r[j] = a[j];
+    int i = 8;
+    for (; i < n - n % 8; i += 8) {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) r[j] = __fadd_rn(r[j], a[i + j]);
+    }
+    float res = __fadd_rn(__fadd_rn(__fadd_rn(r[0], r[1]), __fadd_rn(r[2], r[3])),
+                          __fadd_rn(__fadd_rn(r[4], r[5]), __fadd_rn(r[6], r[7])));
+    for (; i < n; ++i) res = __fadd_rn(res, a[i]);
+    return res;
+}
+
+// pairwise_sum(a, n) without recursion: a stack of pending right halves; bit s of `done` says that the
+// left half of frame s is summed (in left[s]) and the value in hand is its right half.
+__device__ float pairwise_sum(const float *a, int64_t n)
+{
+    int64_t r_off[32], r_n[32];        // n < 2^31 splits fewer than 25 times
+    float left[32];
+    unsigned done = 0;
+    int sp = 0;
+    int64_t off = 0, m = n;
+    for (;;) {
+        while (m > kPwBlock) {
+            const int64_t h = pairwise_split(m);
+            r_off[sp] = off + h; r_n[sp] = m - h; done &= ~(1u << sp); ++sp;
+            m = h;
+        }
+        float v = pairwise_leaf(a + off, (int)m);
+        while (sp > 0 && (done >> (sp - 1) & 1u)) { --sp; v = __fadd_rn(left[sp], v); }
+        if (sp == 0) return v;
+        left[sp - 1] = v; done |= 1u << (sp - 1);
+        off = r_off[sp - 1]; m = r_n[sp - 1];
+    }
+}
+
+// col[i] = the value of member i (members in list order, so cluster k is col[start[k], start[k] + total[k])).
+__global__ void __launch_bounds__(256)
+ordered_column_kernel(const float *__restrict__ data, const int32_t *__restrict__ members, const int64_t *__restrict__ start,
+                      const int64_t *__restrict__ total, int K, float *__restrict__ col, int phase)
+{
+    const int64_t n_members = start[K - 1] + total[K - 1];
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_members; i += (int64_t)gridDim.x * blockDim.x) {
+        int lo = 0, hi = K - 1;                              // the last cluster starting at or before i holds it
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (start[mid] <= i) lo = mid;
+            else hi = mid - 1;
+        }
+        if (in_phase(phase, total[lo], n_members)) col[i] = __ldg(data + members[i]);
+    }
+}
+
+// One block per cluster.  Thread j walks the top kPwLevels levels of the cluster's tree along the bits of j
+// (most significant first, 1 = right half) and sums the node it reaches; a path that meets a leaf early
+// stops there, and only the thread whose remaining bits are zero owns that leaf.  The owners' sums are
+// then combined bottom up, left + right, in shared memory.
+__global__ void __launch_bounds__(kPwThreads)
+ordered_pairwise_kernel(const float *__restrict__ col, const int64_t *__restrict__ start, const int64_t *__restrict__ total,
+                        int K, const float *__restrict__ old_c, float *__restrict__ new_c, int phase)
+{
+    __shared__ float part[kPwThreads];
+    const int k = blockIdx.x, j = threadIdx.x;
+    const int64_t n = total[k];
+    if (!in_phase(phase, n, start[K - 1] + total[K - 1])) return;
+    if (n == 0) {
+        if (j == 0) new_c[k] = old_c[k];                     // km:126 else-branch
+        return;
+    }
+    int64_t off = start[k], m = n;
+    int depth = 0;                                           // the nodes above `depth` on j's path are split
+    for (; depth < kPwLevels && m > kPwBlock; ++depth) {
+        const int64_t h = pairwise_split(m);
+        if ((j >> (kPwLevels - 1 - depth)) & 1) { off += h; m -= h; }
+        else m = h;
+    }
+    const bool owner = (j & ((1 << (kPwLevels - depth)) - 1)) == 0;
+    if (owner) part[j] = pairwise_sum(col + off, m);
+    for (int l = kPwLevels - 1; l >= 0; --l) {               // the node at depth l on j's path: children at j, j + step
+        __syncthreads();
+        const int step = 1 << (kPwLevels - 1 - l);
+        if (owner && (j & (2 * step - 1)) == 0 && l < depth) part[j] = __fadd_rn(part[j], part[j + step]);
+    }
+    if (j == 0) new_c[k] = (float)((double)__fadd_rn(0.0f, part[0]) / (double)n);   // the reduction's identity, then the mean
+}
+
 __global__ void __launch_bounds__(256)
 shift_kernel(const float *__restrict__ a, const float *__restrict__ b, int n, float *__restrict__ shift,
              const int *__restrict__ bad_label)
@@ -297,7 +417,7 @@ static OrdWs ordered_layout(int64_t N, int D, int K)
 {
     OrdWs o;
     const size_t n_tiles = (size_t)((N + kOrdTile - 1) / kOrdTile);
-    size_t off = 256;
+    size_t off = 256;                // [0, 256) of the aligned base: the header (out-of-range flag, big-cluster count)
     o.tile_counts = off; off += align_up(n_tiles * K * sizeof(int32_t), 256);
     o.total = off;       off += align_up((size_t)K * sizeof(int64_t), 256);
     o.start = off;       off += align_up((size_t)K * sizeof(int64_t), 256);
@@ -307,7 +427,7 @@ static OrdWs ordered_layout(int64_t N, int D, int K)
     // aligned sources; the slot count is padded so that every chunk starts on a 256-byte boundary)
     o.slots_pad = align_up((size_t)(N > 0 ? N : 1) + 4 * (size_t)K, 4);      // every cluster padded to whole groups of four
     o.rows32 = off;      off += align_up((size_t)((D + 31) / 32) * o.slots_pad * 32 * sizeof(float), 256);
-    o.bytes = off;
+    o.bytes = off + 256;             // + slack for aligning the caller's pointer to 256 bytes
     return o;
 }
 
@@ -350,14 +470,15 @@ extern "C" int gsl_kmeans_update_ordered(const float *data, const int32_t *label
     const OrdWs L = ordered_layout(N, D, K);
     if (ws_bytes < L.bytes) return fail(GSL_EWORKSPACE, "gsl_kmeans_update_ordered: workspace %zu < %zu", ws_bytes, L.bytes);
     unsigned char *base = reinterpret_cast<unsigned char *>(((uintptr_t)ws + 255) & ~(uintptr_t)255);
-    int32_t *tile_counts = reinterpret_cast<int32_t *>(base + L.tile_counts - 256);
-    int64_t *total = reinterpret_cast<int64_t *>(base + L.total - 256);
-    int64_t *start = reinterpret_cast<int64_t *>(base + L.start - 256);
-    int64_t *pstart = reinterpret_cast<int64_t *>(base + L.pstart - 256);
-    int32_t *members = reinterpret_cast<int32_t *>(base + L.members - 256);
+    int32_t *tile_counts = reinterpret_cast<int32_t *>(base + L.tile_counts);
+    int64_t *total = reinterpret_cast<int64_t *>(base + L.total);
+    int64_t *start = reinterpret_cast<int64_t *>(base + L.start);
+    int64_t *pstart = reinterpret_cast<int64_t *>(base + L.pstart);
+    int32_t *members = reinterpret_cast<int32_t *>(base + L.members);
     const int n_tiles = (int)((N + kOrdTile - 1) / kOrdTile);
     int *bad_label = reinterpret_cast<int *>(base);          // first word of the workspace header
-    GSL_CUDA_TRY(cudaMemsetAsync(bad_label, 0, sizeof(int), st));
+    int *n_big = bad_label + 1;                              // second word: clusters chained on the helper stream
+    GSL_CUDA_TRY(cudaMemsetAsync(bad_label, 0, 2 * sizeof(int), st));
 
     if (N == 0) {
         GSL_CUDA_TRY(cudaMemsetAsync(total, 0, sizeof(int64_t) * (size_t)K, st));
@@ -368,7 +489,7 @@ extern "C" int gsl_kmeans_update_ordered(const float *data, const int32_t *label
         GSL_LAUNCH_CHECK("ordered_count_kernel");
         ordered_scan_kernel<<<K, kOrdThreads, 0, st>>>(tile_counts, n_tiles, K, total);
         GSL_LAUNCH_CHECK("ordered_scan_kernel");
-        ordered_start_kernel<<<1, 32, 0, st>>>(total, K, start, pstart);
+        ordered_start_kernel<<<1, 32, 0, st>>>(total, K, start, pstart, n_big);
         GSL_LAUNCH_CHECK("ordered_start_kernel");
         const size_t sc_smem = (size_t)(8 * K + ((8 * K) & 1)) * sizeof(int) + (size_t)8 * K * sizeof(int64_t);
         GSL_CUDA_TRY(cudaFuncSetAttribute(ordered_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sc_smem));
@@ -376,18 +497,28 @@ extern "C" int gsl_kmeans_update_ordered(const float *data, const int32_t *label
         GSL_LAUNCH_CHECK("ordered_scatter_kernel");
     }
     const dim3 grid((unsigned)K, (unsigned)((D + 31) / 32));
-    float *rows32 = reinterpret_cast<float *>(base + L.rows32 - 256);
+    float *rows32 = reinterpret_cast<float *>(base + L.rows32);
     const size_t st_smem = (size_t)kStreamStages * kStreamRows * 32 * sizeof(float);
     GSL_CUDA_TRY(cudaFuncSetAttribute(ordered_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)st_smem));
     const int64_t warps = (N + 3) / 4 + K;
     const unsigned g = (unsigned)std::min<int64_t>((warps * 32 + 255) / 256, (int64_t)sm_count() * 16);
     auto gather = [&](int phase, cudaStream_t s) -> int {
         if (N == 0) return GSL_OK;
+        if (D == 1) {                                        // one dense column (N floats) in the rows32 area
+            ordered_column_kernel<<<g, 256, 0, s>>>(data, members, start, total, K, rows32, phase);
+            GSL_LAUNCH_CHECK("ordered_column_kernel");
+            return GSL_OK;
+        }
         ordered_gather_kernel<<<g, 256, 0, s>>>(data, D, (int)grid.y, members, start, pstart, total, K, (int64_t)L.slots_pad, rows32, phase);
         GSL_LAUNCH_CHECK("ordered_gather_kernel");
         return GSL_OK;
     };
     auto chains = [&](int phase, cudaStream_t s) -> int {
+        if (D == 1) {
+            ordered_pairwise_kernel<<<K, kPwThreads, 0, s>>>(rows32, start, total, K, old_centroids, new_centroids, phase);
+            GSL_LAUNCH_CHECK("ordered_pairwise_kernel");
+            return GSL_OK;
+        }
         ordered_stream_kernel<<<grid, 32, st_smem, s>>>(rows32, (int64_t)L.slots_pad, D, K, start, pstart, total, old_centroids, new_centroids, phase);
         GSL_LAUNCH_CHECK("ordered_stream_kernel");
         return GSL_OK;

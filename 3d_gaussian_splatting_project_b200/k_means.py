@@ -14,8 +14,9 @@ Semantics kept from the reference (line numbers are the reference's):
     COLORS[c % 8] (divided by 255.0 only in k_means_with_color, :100 vs :148).
 
 `update=` selects how the mean is formed:
-  "ordered" (default on one GPU)  float32 sequential sum in index order -- NumPy's arithmetic,
-            bit-identical centroids, hence identical trajectories;
+  "ordered" (default on one GPU)  NumPy's arithmetic: a float32 sum from +0.0, sequential in index
+            order for D >= 2 and NumPy's pairwise sum for D = 1; bit-identical centroids, hence
+            identical trajectories;
   "fast"    float64 segmented sums, shardable; centroids agree with the reference to its own
             float32 rounding (about 1e-5 relative on clusters of 1e5 members).
 Under torch.distributed (world size > 1) `lloyd` is the sharded entry point: each rank passes ITS

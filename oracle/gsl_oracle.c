@@ -220,11 +220,40 @@ void orc_kmeans_assign(const float *data, int64_t N, int D, const float *centroi
 }
 
 /*
+ * NumPy's pairwise_sum (numpy/_core/src/umath/loops_utils.h.src) of x[0..n), float32 throughout:
+ * plain adds below 8 values, eight strided accumulators up to 128 values, and above that the sum
+ * of the two halves split at n/2 rounded down to a multiple of 8.
+ */
+static float pairwise_sum_f32(const float *x, int64_t n)
+{
+    if (n < 8) {
+        float res = 0.f;
+        for (int64_t i = 0; i < n; ++i) res = res + x[i];
+        return res;
+    }
+    if (n <= 128) {
+        float r[8];
+        int64_t i;
+        for (int j = 0; j < 8; ++j) r[j] = x[j];
+        for (i = 8; i < n - (n % 8); i += 8)
+            for (int j = 0; j < 8; ++j) r[j] = r[j] + x[i + j];
+        float res = ((r[0] + r[1]) + (r[2] + r[3])) + ((r[4] + r[5]) + (r[6] + r[7]));
+        for (; i < n; ++i) res = res + x[i];
+        return res;
+    }
+    int64_t n2 = n / 2;
+    n2 -= n2 % 8;
+    return pairwise_sum_f32(x, n2) + pairwise_sum_f32(x + n2, n - n2);
+}
+
+/*
  * Update step (k_means.py:125-128): data[labels == c].mean(axis=0), else the old centroid.
- * NumPy reduces axis 0 of the gathered float32 [n, D] block row by row, so every column is
- * a float32 sequential sum in index order.  np.mean then calls true_divide(sum_f32,
- * np.intp(n), out=sum_f32, casting='unsafe'): the quotient is formed in float64 and cast
- * back to float32 (numpy/_core/_methods.py:_mean).
+ * NumPy's add.reduce starts every column from its identity +0.0 (so a column of -0.0 sums to
+ * +0.0).  For D >= 2 it reduces axis 0 of the gathered float32 [n, D] block row by row: every
+ * column is a float32 sequential sum in index order.  For D = 1 the reduced axis is contiguous
+ * and the whole column goes through one pairwise_sum.  np.mean then calls true_divide(sum_f32,
+ * np.intp(n), out=sum_f32, casting='unsafe'): the quotient is formed in float64 and cast back to
+ * float32 (numpy/_core/_methods.py:_mean).
  * counts (int64[K], optional) receives the member counts.
  */
 void orc_kmeans_update(const float *data, const int64_t *labels, int64_t N, int D, int K,
@@ -235,12 +264,21 @@ void orc_kmeans_update(const float *data, const int64_t *labels, int64_t N, int 
         float *sum = new_centroids + (int64_t)c * D;
         int64_t n = 0;
         for (int d = 0; d < D; ++d) sum[d] = 0.f;
-        for (int64_t i = 0; i < N; ++i) {
-            if (labels[i] != c) continue;
-            const float *x = data + i * (int64_t)D;
-            if (n == 0) for (int d = 0; d < D; ++d) sum[d] = x[d];
-            else for (int d = 0; d < D; ++d) sum[d] = sum[d] + x[d];
-            ++n;
+        if (D == 1) {
+            for (int64_t i = 0; i < N; ++i) n += labels[i] == c;
+            float *col = n ? (float *)malloc((size_t)n * sizeof(float)) : NULL;
+            int64_t m = 0;
+            for (int64_t i = 0; i < N && col; ++i)
+                if (labels[i] == c) col[m++] = data[i];
+            if (n) sum[0] = 0.f + pairwise_sum_f32(col, n);
+            free(col);
+        } else {
+            for (int64_t i = 0; i < N; ++i) {
+                if (labels[i] != c) continue;
+                const float *x = data + i * (int64_t)D;
+                for (int d = 0; d < D; ++d) sum[d] = sum[d] + x[d];
+                ++n;
+            }
         }
         if (n == 0) {
             for (int d = 0; d < D; ++d) sum[d] = old_centroids[(int64_t)c * D + d];

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 import torch
 
-from util import KMEANS_CASES, load_kmeans_case, pkg
+from util import KMEANS_CASES, assert_bits_equal, load_kmeans_case, pkg
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -81,7 +81,7 @@ def test_step_locked_assignment_and_updates(oracle, n, d, k):
     new_fast, shift_fast = ops.kmeans_finalize(sums, dev(cen))
     new_ord, shift_ord = ops.kmeans_update_ordered(dev(data), lab, dev(cen))
     ref_new, _ = oracle.kmeans_update(data, want, cen)
-    assert np.array_equal(new_ord.cpu().numpy(), ref_new), "ordered update not bit-exact"
+    assert_bits_equal(new_ord.cpu().numpy(), ref_new, "ordered update")
     nf = new_fast.cpu().numpy()
     assert np.allclose(nf, exact.astype(np.float32), rtol=0, atol=0) or np.abs(nf - exact).max() <= 1e-7 * np.abs(exact).max()
     scale = np.abs(ref_new).max(axis=1)
@@ -228,7 +228,7 @@ def test_c5_shape_subsample_step_locked(oracle):
         print(f"[C5 1.5M it{it}] ties {int((gap == 0).sum())}, mismatches {int(bad.sum())}, largest cluster {counts.max()}, "
               f"fast vs reference f32 mean {rel_ref:.2e}, fast vs exact mean {rel_exact:.2e}")
         assert bad.sum() == 0
-        assert np.array_equal(new_ord, ref_new)
+        assert_bits_equal(new_ord, ref_new, f"ordered update, iteration {it}")
         ref_drift = (np.abs(ref_new - exact).max(axis=1) / scale).max()      # the reference's own float32 accumulation error
         print(f"[C5 1.5M it{it}] reference f32 mean vs exact mean {ref_drift:.2e}")
         # north_star asks for 1e-5 against the reference.  The fast update is the exact mean rounded once

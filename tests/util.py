@@ -38,6 +38,17 @@ def blobs(rng, n, spread=0.3):
     return (centres[rng.integers(0, 10, n)] + rng.normal(0, spread, size=(n, 3))).astype(np.float32)
 
 
+def assert_bits_equal(got, want, what="centroids"):
+    """float32 arrays equal bit for bit, so -0.0 != +0.0.  Any two NaNs count as equal: the GPU writes a
+    canonical NaN where x86 keeps the payload and sign of an operand."""
+    got, want = np.asarray(got, np.float32), np.asarray(want, np.float32)
+    assert got.shape == want.shape, (what, got.shape, want.shape)
+    bad = (got.view(np.uint32) != want.view(np.uint32)) & ~(np.isnan(got) & np.isnan(want))
+    if bad.any():
+        first = [(tuple(int(j) for j in i), got[tuple(i)], want[tuple(i)]) for i in np.argwhere(bad)[:4]]
+        raise AssertionError(f"{what}: {int(bad.sum())} of {bad.size} values differ in their bits; (index, got, want): {first}")
+
+
 def load_kmeans_case(name):
     z = np.load(os.path.join(GOLDEN, name + ".npz"))
     d = {k: z[k] for k in z.files}
