@@ -59,7 +59,25 @@ __device__ __forceinline__ float screen_bound(float nx, float nx_term, float ea,
     return fmaf(nx, ea, eb) + nx_term;
 }
 
-// Stages B and C for one row: candidates given as a bit mask over k.
+// The row-wide bound B = screen_bound(nx, ., ea_max, eb_max) holds only where stage A's float32
+// arithmetic neither overflows nor underflows.  B >= 2^-21 (|x'|^2 + max|c'_k|^2) and
+// B >= 1.5 * 2^-9 |x'| max|c'_k|, so:
+//   B < 2^104   ->  |x'|^2, |c'_k|^2 < 2^125 and |x'| |c'_k| < 2^113: no product, dot product,
+//                   |c'_k|^2 or g_k comes near FLT_MAX (~2^128), whatever the TF32 rounding;
+//   B >= 2^-80  ->  max(|x'|, |c'_k|) >= 2^-29.5: subnormal products, operands flushed to zero by
+//                   the tensor cores and the absolute rounding of subnormal partial sums add up to
+//                   less than 2^-120 + 2^-123 max(|x'|, |c'_k|) < 2^-40 B.
+// Rows outside that range (and NaN/Inf rows, whose B is not finite) take every centroid.
+__device__ __forceinline__ bool screen_in_range(float bnd)
+{
+    return bnd >= 0x1p-80f && bnd < 0x1p104f;
+}
+
+// Stages B and C for one row: candidates given as a bit mask over k.  A float32 distance that
+// overflowed (s = +inf) needs no special case: s1 (1 + eps) is finite only for s1 < FLT_MAX / (1 + eps),
+// and eps exceeds the sum's real error, so such a candidate is really farther than the band; when
+// s1 (1 + eps) overflows, the row is not decided in float32 and the band (bound = +inf) keeps every
+// candidate.  Rows with s1 <= 1e-30 (subnormal partial sums) go to float64 with every candidate.
 __device__ __forceinline__ int refine_row(unsigned long long mask, const float *__restrict__ x,
                                           const float *__restrict__ centroids, int D, float eps)
 {

@@ -13,13 +13,16 @@
 //      for the accumulation; second term: rounding of the centring itself).  The kernel uses the
 //      row-wide bound E = max_k E_k (one value per row instead of one per pair):  candidates =
 //      { k : g_k <= min_j g_j + 2 E }, a superset of { k : g_k - E_k <= min_j (g_j + E_j) }.
-//      Typically one or two per row.
+//      Typically one or two per row.  The bound is proven only where stage A's float32 arithmetic
+//      neither overflows nor underflows; rows outside that range take every centroid
+//      (screen_in_range, kmeans_screen.cuh).
 //   B  CUDA cores, candidates only: float32 sum of (x-c)^2 on the original values, relative
 //      error (D + 3) 2^-24; decided when the two smallest differ by more than that.
 //   C  float64, near ties only: scipy-order distance, lowest index first.
 //
 // gsl_kmeans_screen_selftest measures stage A's bound on real data: for every (row, k) it
-// compares (g_k - g_0) with the float64 (d2_k - d2_0) and counts violations of E_k + E_0.
+// compares (g_k - g_0) with the float64 (d2_k - d2_0) and counts violations of E_k + E_0; rows
+// outside screen_in_range are counted apart, not checked.
 //
 // The per-cluster float64 sums that follow are the shared segmented reduction
 // (kmeans_common.cuh).  Compiled with -fmad=false.
@@ -178,7 +181,7 @@ kmeans_step_tc_kernel(const float *__restrict__ data, int64_t N, int D, const fl
     if (kAccumulate)
         for (int i = t; i < K * (D + 1); i += kTcThreads) acc[i] = 0.0;
     const unsigned long long kmask = K >= 64 ? ~0ull : ((1ull << K) - 1ull);
-    unsigned long long n_viol = 0, n_cand = 0;
+    unsigned long long n_viol = 0, n_cand = 0, n_skip = 0;
 
     // Tiles arrive by TMA bulk copy: full 256-row tiles of a 16-byte aligned matrix are one
     // cp.async.bulk each (no staging instructions, no registers); the copy of the NEXT tile is
@@ -222,7 +225,8 @@ kmeans_step_tc_kernel(const float *__restrict__ data, int64_t N, int D, const fl
                     gmin = fminf(gmin, fminf(so.g[mt][j][2 * h], so.g[mt][j][2 * h + 1]));
                 gmin = fminf(gmin, __shfl_xor_sync(0xffffffffu, gmin, 1));
                 gmin = fminf(gmin, __shfl_xor_sync(0xffffffffu, gmin, 2));
-                const float thr = gmin + 2.f * (screen_bound(nx, nx_term, ea_max, eb_max) * 1.000001f);
+                const float bnd = screen_bound(nx, nx_term, ea_max, eb_max);
+                const float thr = gmin + 2.f * (bnd * 1.000001f);
                 unsigned m_lo = 0, m_hi = 0;
 #pragma unroll
                 for (int j = 0; j < 8; ++j)
@@ -235,7 +239,10 @@ kmeans_step_tc_kernel(const float *__restrict__ data, int64_t N, int D, const fl
                 m_lo |= __shfl_xor_sync(0xffffffffu, m_lo, 1); m_hi |= __shfl_xor_sync(0xffffffffu, m_hi, 1);
                 m_lo |= __shfl_xor_sync(0xffffffffu, m_lo, 2); m_hi |= __shfl_xor_sync(0xffffffffu, m_hi, 2);
                 unsigned long long mask = (((unsigned long long)m_hi << 32) | m_lo) & kmask;
-                if (mask == 0 || !(nx < INFINITY)) mask = kmask;   // NaN/Inf/overflowing rows: everything is a candidate
+                // rows outside the range where the bound is proven (screen_in_range), and NaN/Inf rows:
+                // everything is a candidate
+                const bool in_range = screen_in_range(bnd);
+                if (mask == 0 || !in_range) mask = kmask;
                 if (tq == 0) maskbuf[warp * 32 + mt * 16 + g + 8 * h] = mask;
 
                 if (kCheck) {
@@ -243,7 +250,8 @@ kmeans_step_tc_kernel(const float *__restrict__ data, int64_t N, int D, const fl
                     const int r = warp * 32 + mt * 16 + g + 8 * h;
                     const float g0 = __shfl_sync(0xffffffffu, so.g[mt][0][2 * h], lane & ~3);
                     const float e0 = screen_bound(nx, nx_term, eab[0], eab[1]);
-                    if (r < rows) {
+                    if (r < rows && !in_range && tq == 0) ++n_skip;
+                    if (r < rows && in_range) {
                         const float *x = tile + r * pitch;
                         const double d0 = sqdist_scipy(centroids, x, D);
 #pragma unroll
@@ -298,6 +306,7 @@ kmeans_step_tc_kernel(const float *__restrict__ data, int64_t N, int D, const fl
     if (kCheck) {
         atomicAdd(check_out, n_viol);
         atomicAdd(check_out + 1, n_cand);
+        atomicAdd(check_out + 2, n_skip);
     }
 }
 
@@ -332,12 +341,12 @@ int launch_step_tc(bool accumulate, const float *data, int64_t N, int D, const f
 using namespace gsl;
 
 extern "C" int gsl_kmeans_screen_selftest(const float *data, int64_t N, int D, const float *centroids, int K,
-                                          int32_t *labels, unsigned long long *out2, void *stream)
+                                          int32_t *labels, unsigned long long *out3, void *stream)
 {
-    if (!data || !centroids || !labels || !out2 || N < 0) return fail(GSL_EINVAL, "gsl_kmeans_screen_selftest: bad argument");
+    if (!data || !centroids || !labels || !out3 || N < 0) return fail(GSL_EINVAL, "gsl_kmeans_screen_selftest: bad argument");
     if (!tc_supported(D, K)) return fail(GSL_EINVAL, "gsl_kmeans_screen_selftest: needs K <= 64 and 8 <= D <= 64");
     if (N == 0) return GSL_OK;
     const int64_t tiles = (N + kTcRows - 1) / kTcRows;
     const int64_t cap = (int64_t)sm_count() * 2;
-    return launch_tc_t<false, true>(data, N, D, centroids, K, labels, nullptr, (int)(tiles < cap ? tiles : cap), out2, (cudaStream_t)stream);
+    return launch_tc_t<false, true>(data, N, D, centroids, K, labels, nullptr, (int)(tiles < cap ? tiles : cap), out3, (cudaStream_t)stream);
 }

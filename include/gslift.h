@@ -257,12 +257,14 @@ int gsl_kmeans_update_ordered(const float *data, const int32_t *labels, int64_t 
 /*
  * Test hook for the tensor-core screening of gsl_kmeans_assign/step (K <= 64, 8 <= D <= 64):
  * runs the assignment and, for every (row, centroid), compares the screened ranking value with
- * the float64 distance.  out2[0] += number of (row, centroid) pairs whose error exceeds the
- * bound the kernel relies on (must stay 0); out2[1] += total candidates forwarded to the
- * float32/float64 stages.  out2 is a device array the caller zeroes.
+ * the float64 distance.  out3[0] += number of (row, centroid) pairs whose error exceeds the
+ * bound the kernel relies on (must stay 0); out3[1] += total candidates forwarded to the
+ * float32/float64 stages; out3[2] += rows outside the range where the bound is proven (values
+ * near float32 overflow or underflow, NaN/Inf): they take every centroid as a candidate and are
+ * not checked.  out3 is a device array of three counters the caller zeroes.
  */
 int gsl_kmeans_screen_selftest(const float *data, int64_t N, int D, const float *centroids, int K,
-                               int32_t *labels, unsigned long long *out2, void *stream);
+                               int32_t *labels, unsigned long long *out3, void *stream);
 
 /* Recolouring (km:99-101, :147-149): colors[i][0..3) = palette[labels[i] % 8]; `palette` is a
  * device float32 [8][3] the host fills with COLORS (km:8), divided by 255.0 or not. */

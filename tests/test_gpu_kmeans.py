@@ -151,15 +151,16 @@ def test_tensor_core_screening_bound_holds_on_data():
     wide = (rng.standard_normal((100_000, 8)) * np.array([1e-3, 1, 1e3, 1, 1, 1e2, 1, 1e-2])).astype(np.float32)
     sets.append(("mixed scales D=8", wide, wide[rng.choice(len(wide), 16, replace=False)]))
     for name, x, c in sets:
-        out = torch.zeros(2, dtype=torch.int64, device=DEV)
+        out = torch.zeros(3, dtype=torch.int64, device=DEV)
         labels = torch.empty(len(x), dtype=torch.int32, device=DEV)
         dx, dc = dev(x), dev(c)
         native.check(native.lib().gsl_kmeans_screen_selftest(dx.data_ptr(), len(x), x.shape[1], dc.data_ptr(), len(c),
                                                              labels.data_ptr(), out.data_ptr(), None))
         torch.cuda.synchronize()
-        viol, cand = (int(v) for v in out.tolist())
+        viol, cand, skip = (int(v) for v in out.tolist())
         print(f"[tc screen] {name}: bound violations {viol}, candidates per row {cand / len(x):.3f}")
         assert viol == 0
+        assert skip == 0, "ordinary data must stay inside the range where the bound is proven"
 
 
 def test_ties_duplicates_and_determinism(oracle):
