@@ -47,7 +47,7 @@ constexpr int kDigitBits = 10;
 constexpr int kDigits = 1 << kDigitBits;
 constexpr int kWarps = 8;
 constexpr int kMaxRanges = 343;            // (2 * 3 + 1)^3 cells
-constexpr int kMaxList = 64;               // neighbour lists are returned for k <= 64
+constexpr int kMaxList = 64;               // lists of k <= 64 are ordered inside knn_pca_kernel, longer ones by knn_order_kernel
 constexpr int kBucketCap = 256;            // candidates of the k-th value's histogram bucket resolved in shared memory
 
 struct BucketEntry {                       // 16 bytes: kBucketCap of them reuse the 4 KB of the histogram
@@ -269,7 +269,7 @@ struct QueryOut {
     const double *normals_in;  // [N][3] normals for the residual, may be NULL (then the computed one)
     double *residuals;         // [N] out, may be NULL
     double *centroids;         // [N][3] out, may be NULL
-    int32_t *knn;              // [N][k] out, k <= kMaxList, may be NULL
+    int32_t *knn;              // [N][k] out, k <= GSL_REGION_MAX_LIST, may be NULL
 };
 
 struct WarpScratch {
@@ -422,6 +422,9 @@ __device__ __forceinline__ double warp_sum(double v)
     return v;
 }
 
+// kLongList: the caller asked for lists of k > 64, written straight out in walk order (a separate
+// instantiation, so that the other calls run the code they always ran)
+template <bool kLongList>
 __global__ void __launch_bounds__(kWarps * 32, 3) knn_pca_kernel(const float4 *__restrict__ sorted, int64_t N, int k,
                                                               const GridInfo *__restrict__ ginfo, Tables T, QueryOut out,
                                                               unsigned long long *__restrict__ stats)
@@ -581,6 +584,7 @@ __global__ void __launch_bounds__(kWarps * 32, 3) knn_pca_kernel(const float4 *_
         double s1[3] = {0, 0, 0}, s2[6] = {0, 0, 0, 0, 0, 0};
         int n_list = 0;
         const bool want_list = out.knn != nullptr;
+        constexpr bool emit = kLongList;                  // k > 64: the list goes out in walk order, knn_order_kernel sorts it
         auto take = [&](bool sel, const float4 p, double d2) {
             if (sel) {
                 const double dx = __dsub_rn((double)p.x, qx), dy = __dsub_rn((double)p.y, qy), dz = __dsub_rn((double)p.z, qz);
@@ -592,7 +596,9 @@ __global__ void __launch_bounds__(kWarps * 32, 3) knn_pca_kernel(const float4 *_
                 const unsigned m = __ballot_sync(0xffffffffu, sel);
                 if (sel) {
                     const int at = n_list + __popc(m & radix::lanemask_lt());
-                    if (at < kMaxList) {
+                    if (emit) {
+                        if (at < k) out.knn[(size_t)q_index * k + at] = (int32_t)__float_as_uint(p.w);
+                    } else if (at < kMaxList) {
                         sc.list_d[at] = d2;
                         sc.list_i[at] = __float_as_uint(p.w);
                     }
@@ -698,7 +704,7 @@ __global__ void __launch_bounds__(kWarps * 32, 3) knn_pca_kernel(const float4 *_
             }
             if (lane == 0) out.residuals[q_index] = fabs(-(nrm[0] * mx + nrm[1] * my + nrm[2] * mz));    // rg:161
         }
-        if (want_list) {
+        if (want_list && !emit) {
             // order the k <= 64 selected neighbours by (distance, index): rank sort in shared memory
             __syncwarp();
             const int n = min(n_list, kMaxList);
@@ -720,6 +726,64 @@ __global__ void __launch_bounds__(kWarps * 32, 3) knn_pca_kernel(const float4 *_
             atomicAdd(&stats[2], n_failed);
             atomicAdd(&stats[3], n_select);
         }
+    }
+}
+
+// Lists of k > 64 leave knn_pca_kernel in walk order.  This kernel puts every row into increasing
+// (distance, index) order, KDTree.query's: the key of a neighbour is the float64 bit pattern of its
+// squared distance (recomputed from pos with the selector's own sqdist, monotone for d2 >= 0) and its
+// index, so keys are unique and the order is a total one.  A row's keys, padded to a power of two P
+// with +inf sentinels, are bitonic-sorted in shared memory; rows of small k share a CTA.
+constexpr int kOrderThreads = 256;
+constexpr int kOrderMinKeys = 2048;        // keys per CTA: rows of P < 2048 share one
+constexpr int kOrderKeyBytes = 12;         // 8-byte distance bits + 4-byte index
+static_assert((size_t)GSL_REGION_MAX_LIST * kOrderKeyBytes <= 227 * 1024, "a row of keys fits one CTA's shared memory");
+
+__global__ void __launch_bounds__(kOrderThreads) knn_order_kernel(const float *__restrict__ pos, int64_t N, int k, int log_p,
+                                                                  int rows_per_cta, int32_t *__restrict__ knn)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int P = 1 << log_p, keys = P * rows_per_cta;
+    unsigned long long *kd = reinterpret_cast<unsigned long long *>(smem_raw);
+    uint32_t *ki = reinterpret_cast<uint32_t *>(kd + keys);
+    const int64_t row0 = (int64_t)blockIdx.x * rows_per_cta;
+    for (int t = threadIdx.x; t < keys; t += kOrderThreads) {
+        const int64_t row = row0 + (t >> log_p);
+        const int i = t & (P - 1);
+        unsigned long long d = 0x7ff0000000000000ull;          // +inf: every real d2 of finite float32 points is finite
+        uint32_t j = 0xffffffffu;
+        if (row < N && i < k) {
+            j = (uint32_t)knn[(size_t)row * k + i];
+            const float4 p = make_float4(pos[3 * (size_t)j], pos[3 * (size_t)j + 1], pos[3 * (size_t)j + 2], 0.f);
+            d = (unsigned long long)__double_as_longlong(
+                sqdist(p, (double)pos[3 * (size_t)row], (double)pos[3 * (size_t)row + 1], (double)pos[3 * (size_t)row + 2]));
+        }
+        kd[t] = d;
+        ki[t] = j;
+    }
+    const int half = keys >> 1;
+    for (int size = 2; size <= P; size <<= 1)
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            __syncthreads();
+            for (int t = threadIdx.x; t < half; t += kOrderThreads) {
+                // pair t: rows hold P / 2 pairs each; within a row, a = the lower element of the pair
+                const int r = t >> (log_p - 1), i = t & ((P >> 1) - 1);
+                const int a = ((i & ~(stride - 1)) << 1) | (i & (stride - 1));
+                const int ga = (r << log_p) + a, gb = ga + stride;
+                const unsigned long long da = kd[ga], db = kd[gb];
+                const uint32_t ia = ki[ga], ib = ki[gb];
+                const bool a_after_b = da > db || (da == db && ia > ib);
+                if (a_after_b == ((a & size) == 0)) {          // ascending runs where bit `size` of a is clear
+                    kd[ga] = db; kd[gb] = da;
+                    ki[ga] = ib; ki[gb] = ia;
+                }
+            }
+        }
+    __syncthreads();
+    for (int t = threadIdx.x; t < keys; t += kOrderThreads) {
+        const int64_t row = row0 + (t >> log_p);
+        const int i = t & (P - 1);
+        if (row < N && i < k) knn[(size_t)row * k + i] = (int32_t)ki[t];
     }
 }
 
@@ -763,7 +827,9 @@ extern "C" int gsl_region_knn_pca(const float *pos, int64_t N, int k, const doub
     if (N < 0 || k < 1 || (N > 0 && (!pos || !ws))) return fail(GSL_EINVAL, "gsl_region_knn_pca: bad argument");
     if (N > 0x7fffffffLL) return fail(GSL_EINVAL, "gsl_region_knn_pca: more than 2^31 - 1 points");
     if (k > N && N > 0) return fail(GSL_EINVAL, "gsl_region_knn_pca: k = %d exceeds the number of points %lld", k, (long long)N);
-    if (knn && k > rg::kMaxList) return fail(GSL_EINVAL, "gsl_region_knn_pca: neighbour lists are returned for k <= %d", rg::kMaxList);
+    if (knn && k > GSL_REGION_MAX_LIST)
+        return fail(GSL_EINVAL, "gsl_region_knn_pca: neighbour lists are returned for k <= %d (GSL_REGION_MAX_LIST), k = %d",
+                    GSL_REGION_MAX_LIST, k);
     if (N == 0) return GSL_OK;
     const rg::Plan p = rg::plan(N);
     if (ws_bytes < p.total) return fail(GSL_EWORKSPACE, "gsl_region_knn_pca: workspace %zu < %zu", ws_bytes, p.total);
@@ -809,10 +875,22 @@ extern "C" int gsl_region_knn_pca(const float *pos, int64_t N, int k, const doub
     }
     rg::QueryOut out{normals, normals_in, residuals, centroids, knn};
     const size_t smem = sizeof(rg::WarpScratch) * rg::kWarps;
-    GSL_CUDA_TRY(cudaFuncSetAttribute(rg::knn_pca_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const bool long_list = knn && k > rg::kMaxList;
+    const auto kernel = long_list ? rg::knn_pca_kernel<true> : rg::knn_pca_kernel<false>;
+    GSL_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int qgrid = (int)std::min<int64_t>((N + rg::kWarps - 1) / rg::kWarps, (int64_t)sm_count() * 16);
-    rg::knn_pca_kernel<<<qgrid, rg::kWarps * 32, smem, st>>>(sorted, N, k, ginfo, T, out, stats);
+    kernel<<<qgrid, rg::kWarps * 32, smem, st>>>(sorted, N, k, ginfo, T, out, stats);
     GSL_LAUNCH_CHECK("rg::knn_pca_kernel");
+    if (long_list) {
+        int log_p = 0;
+        while ((1 << log_p) < k) ++log_p;
+        const int rows = std::max(1, rg::kOrderMinKeys >> log_p);
+        const size_t osmem = (size_t)rows * ((size_t)1 << log_p) * rg::kOrderKeyBytes;
+        GSL_CUDA_TRY(cudaFuncSetAttribute(rg::knn_order_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)osmem));
+        const int64_t ogrid = (N + rows - 1) / rows;
+        rg::knn_order_kernel<<<(unsigned)ogrid, rg::kOrderThreads, osmem, st>>>(pos, N, k, log_p, rows, knn);
+        GSL_LAUNCH_CHECK("rg::knn_order_kernel");
+    }
     return GSL_OK;
 }
 

@@ -42,7 +42,8 @@ def _device_points(V1) -> torch.Tensor:
 def knn_pca(V1, k: int, normals_in=None, want_normals=True, want_residuals=True, want_centroids=False,
             want_knn=False, want_stats=False) -> dict:
     """One pass of gsl_region_knn_pca.  Returns device tensors: normals f64 [N,3], residuals f64 [N],
-    centroids f64 [N,3], knn int32 [N,k] (k <= 64), as requested."""
+    centroids f64 [N,3], knn int32 [N,k] in increasing (distance, index) order, as requested.  Lists are
+    returned for k <= GSL_REGION_MAX_LIST (16384); above that want_knn raises the library's GslError."""
     pos = _device_points(V1)
     N = pos.shape[0]
     dev = pos.device

@@ -45,6 +45,8 @@ extern "C" {
                                    255 = the coarse table's "mixed cell" marker)             */
 #define GSL_KMEANS_MAX_K 1024
 #define GSL_KMEANS_MAX_D 256
+#define GSL_REGION_MAX_LIST 16384  /* longest neighbour list gsl_region_knn_pca returns: one row's
+                                      12-byte sort keys fill one CTA's shared memory */
 
 /*
  * One camera view, host side.  Everything project_gaussian (dls:43-82) and the rescale in
@@ -337,7 +339,9 @@ int gsl_viewer_hit_test(const float *pos, const int32_t *labels, int64_t N, int 
  *   normals_in  optional float64 [N][3]: normals to form the residual with (compute_residuals takes
  *               them as an argument, rg:130); NULL = the normals computed by this call
  *   normals     optional float64 [N][3] out        residuals  optional float64 [N] out
- *   centroids   optional float64 [N][3] out        knn        optional int32 [N][k] out, k <= 64:
+ *   centroids   optional float64 [N][3] out
+ *   knn         optional int32 [N][k] out, k <= GSL_REGION_MAX_LIST (larger k with knn != NULL:
+ *               GSL_EINVAL before any device work; the other outputs take any k <= N):
  *               neighbour indices in increasing (distance, index) order (KDTree.query order)
  *   stats       optional uint64 [4], device, caller zeroes: += walks over candidate cells, += points visited by
  *               those walks, += cubes that turned out too small, += walks spent on further select digits
