@@ -123,7 +123,7 @@ def _precomputed_map(output_dir, img_name):
 # ----------------------------------------------------------------------------------------
 # the hot path
 # ----------------------------------------------------------------------------------------
-_copy_streams = {}
+_side_streams = {}                 # per (device, role): the copy stream of the uploads, the push stream of the peer pushes
 last_call_stats = {}               # bytes lift_labels moved over PCIe in its last call (this process)
 _pinned_codes = {}                 # pinned uint8 staging for host-narrowed views (grown to the largest scene seen)
 _host_stage = {"px_per_s": None, "fixed_s": 0.008}   # calibrated by use: host narrowing rate (pixels per second, all
@@ -140,11 +140,11 @@ def _dist():
     return None, 1, 0
 
 
-def _copy_stream(device):
-    key = (device.type, device.index)
-    if key not in _copy_streams:
-        _copy_streams[key] = torch.cuda.Stream(device)
-    return _copy_streams[key]
+def _side_stream(device, role):
+    key = (device.type, device.index, role)
+    if key not in _side_streams:
+        _side_streams[key] = torch.cuda.Stream(device)
+    return _side_streams[key]
 
 
 def _host_cores():
@@ -216,42 +216,106 @@ def _copy_views(seg_maps, sizes, v0, v1, dst):
     return off
 
 
-def _runs(shapes, v0, v1):
-    """(first view, count) of the runs of equal map shapes among views [v0, v1)."""
-    v = v0
-    while v < v1:
-        n = 1
-        while v + n < v1 and shapes[v + n] == shapes[v]:
-            n += 1
-        yield v, n
-        v += n
+def _upload_all(seg_maps, shapes, device):
+    """Every map, uploaded (current stream) as one flat int32 device tensor."""
+    sizes = [h * w for h, w in shapes]
+    staged = torch.empty(int(sum(sizes)), dtype=torch.int32, device=device)
+    _copy_views(seg_maps, sizes, 0, len(seg_maps), staged)
+    return staged
 
 
-class _Staged:
-    """Packed maps on the device plus the code window they were packed with."""
+def _chunk_plan(shapes, host_fraction):
+    """How one process stages its views.  Views [0, v_int32) cross the bus as int32 in chunks of CH;
+    the remaining chunks (round(host_fraction * chunks) of them) are narrowed to 1-byte codes on the
+    host in `batches` of view ranges, two chunks at a time while more than three remain and then one
+    at a time, so that little is left to upload once the host is done.  Returns (v_int32, batches,
+    bytes the maps put on the bus)."""
+    V = len(shapes)
+    n_chunks = -(-V // CH)
+    n_dev = n_chunks - int(round(host_fraction * n_chunks))
+    batches, b0 = [], n_dev
+    while b0 < n_chunks:
+        b1 = b0 + (2 if n_chunks - b0 > 3 else 1)
+        batches.append((b0 * CH, min(b1 * CH, V)))
+        b0 = b1
+    v_int32 = min(n_dev * CH, V)
+    px = [h * w for h, w in shapes]
+    return v_int32, batches, 4 * sum(px[:v_int32]) + sum(px[v_int32:])
 
-    def __init__(self, packed, label_min, n_classes, lo, hi, h2d_bytes, views_as_int32, views_narrowed):
-        self.packed, self.label_min, self.n_classes = packed, label_min, n_classes
-        self.lo, self.hi = lo, hi                      # value range seen in the maps
-        self.h2d_bytes, self.views_as_int32, self.views_narrowed = h2d_bytes, views_as_int32, views_narrowed
+
+def _stage_int32(seg_maps, shapes, sizes, starts, pstarts, device, v_lo, v_hi, packed, before_wait, on_chunk):
+    """Views [v_lo, v_hi) cross the bus as int32 in chunks of CH views, two staging buffers in flight
+    on the copy stream, and are packed on the current stream with the default code window
+    (gsl_pack_labels).  `starts` / `pstarts` are the pixel / packed-byte offsets of every view.
+
+    The first two uploads are enqueued before anything else happens on the host; `before_wait`
+    (the Gaussian ordering, which reads no maps) is called right after them, and `packed` is
+    allocated after it when None.  `on_chunk(v0, v1, packed)`, when given, is called once chunk
+    [v0, v1) has been packed (enqueued on the current stream) and the upload that refills its buffer
+    has been enqueued.  Returns (packed, int32 device tensor [min, max] of the values uploaded)."""
+    from ._native import check, lib
+    L = lib()
+    main = torch.cuda.current_stream(device)
+    copy = _side_stream(device, "copy")
+    copy.wait_stream(main)          # device-resident maps may still be being written; freed blocks may still be in use
+    chunks = list(range(v_lo, v_hi, CH))
+    chunk_px = max([int(starts[min(v0 + CH, v_hi)] - starts[v0]) for v0 in chunks] + [1])
+    with torch.cuda.stream(copy):
+        slots = [torch.empty(chunk_px, dtype=torch.int32, device=device) for _ in range(2)]
+    for sl in slots:
+        sl.record_stream(main)
+    slot_free, ready, n_px = [None, None], [None] * len(chunks), [0] * len(chunks)
+
+    def upload(ci):
+        v0 = chunks[ci]
+        with torch.cuda.stream(copy):
+            if slot_free[ci % 2] is not None:
+                copy.wait_event(slot_free[ci % 2])
+            n_px[ci] = _copy_views(seg_maps, sizes, v0, min(v0 + CH, v_hi), slots[ci % 2])
+            ready[ci] = torch.cuda.Event()
+            ready[ci].record(copy)
+
+    for ci in range(min(2, len(chunks))):                        # the transfer starts now
+        upload(ci)
+    before_wait()
+    if packed is None:
+        packed = torch.empty(int(pstarts[-1]), dtype=torch.uint8, device=device)
+    minmax = torch.tensor([2**31 - 1, -2**31], dtype=torch.int32, device=device)
+    err = torch.zeros(1, dtype=torch.int32, device=device)
+    # everything below is enqueued without waiting
+    for ci, v0 in enumerate(chunks):
+        v1 = min(v0 + CH, v_hi)
+        buf = slots[ci % 2]
+        main.wait_event(ready[ci])
+        check(L.gsl_label_range(buf.data_ptr(), n_px[ci], minmax.data_ptr(), main.cuda_stream))
+        for v, n in ops._runs(shapes, v0, v1):
+            check(L.gsl_pack_labels(buf.data_ptr() + 4 * int(starts[v] - starts[v0]), n, shapes[v][1], shapes[v][0],
+                                    packed.data_ptr() + int(pstarts[v]), ops.DEFAULT_LABEL_MIN, ops.DEFAULT_N_CLASSES,
+                                    err.data_ptr(), main.cuda_stream))
+        slot_free[ci % 2] = torch.cuda.Event()
+        slot_free[ci % 2].record(main)
+        if ci + 2 < len(chunks):
+            upload(ci + 2)                                       # refills the slot just packed
+        if on_chunk is not None:
+            on_chunk(v0, v1, packed)
+    return packed, minmax
 
 
-def _stage_pipelined(seg_maps, shapes, device, before_wait=None, on_packed=None):
+def _stage_single(seg_maps, shapes, device, before_wait, on_packed):
     """One-process staging of HOST (or device) maps, organised around the PCIe transfer, which is
     what such a call waits for (N2 of SURVEY 8f):
 
-      * the first chunks of 16 views cross the bus as int32, two staging buffers in flight on a
-        copy stream, and are packed on the device (gsl_pack_labels);
+      * the first chunks of 16 views cross the bus as int32 and are packed on the device
+        (_stage_int32);
       * the remaining chunks are narrowed to 1-byte codes by the host cores meanwhile
         (gsl_host_pack_labels), cross as uint8 behind the int32 chunks, and are laid out on the
         device (gsl_tile_codes).
 
-    The first uploads are enqueued before anything else happens on the host; `before_wait` (the
-    Gaussian ordering, which reads no maps) is called right after them, and `on_packed(v)` every
-    time the packed maps of views [0, v) have been enqueued on the main stream, so that the caller
-    can sweep them while later maps are still crossing the bus.  Codes are label + 2
-    (label_min = -1, 254 codes); the caller checks the value range and re-stages when the labels do
-    not fit that window."""
+    _chunk_plan makes the split.  `on_packed(v0, v1, packed)` is called every time the packed maps
+    of views [0, v1) have been enqueued on the main stream, so that the caller can sweep them while
+    later maps are still crossing the bus.  Codes are label + 2 (label_min = -1, 254 codes).
+    Returns (packed, lo, hi), the value range seen, which the caller checks, re-staging when the
+    labels do not fit that window."""
     import ctypes
     import time
     from ._native import check, lib
@@ -260,60 +324,15 @@ def _stage_pipelined(seg_maps, shapes, device, before_wait=None, on_packed=None)
     sizes = [h * w for h, w in shapes]
     starts = np.concatenate(([0], np.cumsum(sizes))).astype(np.int64)     # pixels, row-major staging
     pstarts = ops.packed_offsets(shapes)                                   # bytes, packed layout
+    hv0, batches, h2d_bytes = _chunk_plan(shapes, _host_fraction(seg_maps, int(starts[-1])))
     main = torch.cuda.current_stream(device)
-    copy = _copy_stream(device)
-    copy.wait_stream(main)          # device-resident maps may still be being written; freed blocks may still be in use
-    chunks = list(range(0, V, CH))
-    n_host = int(round(_host_fraction(seg_maps, int(starts[-1])) * len(chunks)))
-    n_dev = len(chunks) - n_host                                 # chunks [0, n_dev) cross as int32
-    chunk_px = max([int(starts[min(v0 + CH, V)] - starts[v0]) for v0 in chunks[:n_dev]] + [1])
-    with torch.cuda.stream(copy):
-        slots = [torch.empty(chunk_px, dtype=torch.int32, device=device) for _ in range(2)]
-    for sl in slots:
-        sl.record_stream(main)
-    slot_free = [None, None]
-    ready = [None] * n_dev
-
-    def upload(ci):
-        v0 = chunks[ci]
-        with torch.cuda.stream(copy):
-            if slot_free[ci % 2] is not None:
-                copy.wait_event(slot_free[ci % 2])
-            n = _copy_views(seg_maps, sizes, v0, min(v0 + CH, V), slots[ci % 2])
-            ready[ci] = torch.cuda.Event()
-            ready[ci].record(copy)
-        return n
-
+    copy = _side_stream(device, "copy")
     t_call0 = time.perf_counter()
     with torch.cuda.device(device):
-        n_px = [0] * n_dev
-        for ci in range(min(2, n_dev)):                          # the transfer starts now
-            n_px[ci] = upload(ci)
-        if before_wait is not None:
-            before_wait()
-        packed = torch.empty(int(pstarts[-1]), dtype=torch.uint8, device=device)
-        minmax = torch.tensor([2**31 - 1, -2**31], dtype=torch.int32, device=device)
-        err = torch.zeros(1, dtype=torch.int32, device=device)
-        # ---- chunks that cross as int32: everything below is enqueued without waiting
-        for ci in range(n_dev):
-            v0 = chunks[ci]
-            v1 = min(v0 + CH, V)
-            buf = slots[ci % 2]
-            main.wait_event(ready[ci])
-            check(L.gsl_label_range(buf.data_ptr(), n_px[ci], minmax.data_ptr(), main.cuda_stream))
-            for v, n in _runs(shapes, v0, v1):
-                check(L.gsl_pack_labels(buf.data_ptr() + 4 * int(starts[v] - starts[v0]), n, shapes[v][1], shapes[v][0],
-                                        packed.data_ptr() + int(pstarts[v]), -1, ops.DEFAULT_N_CLASSES, err.data_ptr(), main.cuda_stream))
-            slot_free[ci % 2] = torch.cuda.Event()
-            slot_free[ci % 2].record(main)
-            if ci + 2 < n_dev:
-                n_px[ci + 2] = upload(ci + 2)            # refills the slot just packed
-            if on_packed is not None:
-                on_packed(v1, packed)
-        # ---- chunks narrowed on the host, a few at a time, while the DMA engine is busy with the above
+        packed, minmax = _stage_int32(seg_maps, shapes, sizes, starts, pstarts, device, 0, hv0, None, before_wait, on_packed)
+        # ---- views [hv0, V) narrowed on the host, a batch at a time, while the DMA engine is busy with the above
         host_mm = (ctypes.c_int * 2)(2**31 - 1, -2**31)
-        if n_host:
-            hv0 = chunks[n_dev]
+        if batches:
             host_px = int(starts[V] - starts[hv0])
             if _pinned_codes.get("n", 0) < host_px:
                 # sized for every view of the scene, so that a later call whose calibrated split moves
@@ -327,23 +346,15 @@ def _stage_pipelined(seg_maps, shapes, device, before_wait=None, on_packed=None)
                 codes = torch.empty(host_px, dtype=torch.uint8, device=device)
             codes.record_stream(main)
             bad = ctypes.c_int(0)
-            # host batches of two chunks; the last two chunks go one at a time, so that little is
-            # left to upload once the host is done
-            batches, b0 = [], n_dev
-            while b0 < len(chunks):
-                nb = 2 if len(chunks) - b0 > 3 else 1
-                batches.append((b0, min(b0 + nb, len(chunks))))
-                b0 += nb
             t_narrow, px_narrow = 0.0, 0
-            for b0, b1 in batches:
-                vb0 = chunks[b0]
-                vb1 = min(chunks[b1 - 1] + CH, V)
+            for vb0, vb1 in batches:
                 keep = [_host_ptr(seg_maps[v]) for v in range(vb0, vb1)]
                 ptrs = (ctypes.c_void_p * len(keep))(*[k[0] for k in keep])
                 npx = (ctypes.c_int64 * len(keep))(*[sizes[v] for v in range(vb0, vb1)])
                 off0, off1 = int(starts[vb0] - starts[hv0]), int(starts[vb1] - starts[hv0])
                 t0 = time.perf_counter()
-                check(L.gsl_host_pack_labels(ptrs, npx, len(keep), -1, ops.DEFAULT_N_CLASSES, pinned.data_ptr() + off0, _host_cores(), host_mm, ctypes.byref(bad)))
+                check(L.gsl_host_pack_labels(ptrs, npx, len(keep), ops.DEFAULT_LABEL_MIN, ops.DEFAULT_N_CLASSES,
+                                             pinned.data_ptr() + off0, _host_cores(), host_mm, ctypes.byref(bad)))
                 t_narrow += time.perf_counter() - t0
                 px_narrow += off1 - off0
                 with torch.cuda.stream(copy):
@@ -351,30 +362,26 @@ def _stage_pipelined(seg_maps, shapes, device, before_wait=None, on_packed=None)
                     landed = torch.cuda.Event()
                     landed.record(copy)
                 main.wait_event(landed)
-                for v, n in _runs(shapes, vb0, vb1):
+                for v, n in ops._runs(shapes, vb0, vb1):
                     check(L.gsl_tile_codes(codes.data_ptr() + int(starts[v] - starts[hv0]), n, shapes[v][1], shapes[v][0],
                                            packed.data_ptr() + int(pstarts[v]), main.cuda_stream))
-                if on_packed is not None:
-                    on_packed(vb1, packed)
+                on_packed(vb0, vb1, packed)
             if t_narrow > 0:
                 _host_stage["px_per_s"] = px_narrow / t_narrow
                 # the other host work of this call; first calls also pay allocations, hence the cap
                 _host_stage["fixed_s"] = min(max(time.perf_counter() - t_call0 - t_narrow, 0.0), 0.015)
-        dev_px = int(starts[chunks[n_dev]] if n_dev < len(chunks) else starts[V])
         lo, hi = (int(x) for x in minmax.tolist())           # synchronises: every copy has been consumed
-        lo, hi = min(lo, int(host_mm[0])), max(hi, int(host_mm[1]))
-    return _Staged(packed, -1, ops.DEFAULT_N_CLASSES, lo, hi, 4 * dev_px + int(starts[V] - dev_px), min(n_dev * CH, V), V - min(n_dev * CH, V))
+    last_call_stats.update(h2d_bytes=h2d_bytes, views_as_int32=hv0, views_narrowed_on_host=V - hv0)
+    return packed, min(lo, int(host_mm[0])), max(hi, int(host_mm[1]))
 
 
-def _stage_sharded(seg_maps, shapes, device, dist, world, rank, before_wait=None):
+def _stage_sharded(seg_maps, shapes, device, dist, world, rank, before_wait):
     """Multi-rank staging: every rank holds the same host maps but uploads and packs only its
-    contiguous block of views, chunk by chunk (two int32 staging buffers in flight on a copy
-    stream), and PUSHES every packed chunk straight into all ranks' packed buffers over peer
-    memory (torch symmetric memory = CUDA peer mapping over NVLink) while the next chunk crosses
-    PCIe.  The PCIe cost per rank drops by the world size and no collective library call sits on
-    the data path; one barrier at the end publishes the buffers."""
-    from ._native import check, lib
-    L = lib()
+    contiguous block of views (_stage_int32), and PUSHES every packed chunk straight into all ranks'
+    packed buffers over peer memory (torch symmetric memory = CUDA peer mapping over NVLink) while
+    the next chunk crosses PCIe.  The PCIe cost per rank drops by the world size and no collective
+    library call sits on the data path; one barrier at the end publishes the buffers.
+    Returns (packed, lo, hi) as _stage_single does."""
     V = len(seg_maps)
     sizes = [h * w for h, w in shapes]
     starts = np.concatenate(([0], np.cumsum(sizes))).astype(np.int64)
@@ -384,8 +391,6 @@ def _stage_sharded(seg_maps, shapes, device, dist, world, rank, before_wait=None
     cuts = [r * per + min(r, extra) for r in range(world + 1)]
     v_lo, v_hi = cuts[rank], cuts[rank + 1]
     main = torch.cuda.current_stream(device)
-    copy = _copy_stream(device)
-    copy.wait_stream(main)
     peers = None
     use_symm = os.environ.get("GSLIFT_STAGE_EXCHANGE", "symm") != "nccl"
     if use_symm:
@@ -405,52 +410,22 @@ def _stage_sharded(seg_maps, shapes, device, dist, world, rank, before_wait=None
     else:
         # nobody may still be sweeping the previous call's maps when the pushes of this one arrive
         dist.barrier()
-    chunks = list(range(v_lo, v_hi, CH))
-    chunk_px = max([int(starts[min(v0 + CH, v_hi)] - starts[v0]) for v0 in chunks] + [1])
-    with torch.cuda.stream(copy):
-        slots = [torch.empty(chunk_px, dtype=torch.int32, device=device) for _ in range(2)]
-    for sl in slots:
-        sl.record_stream(main)
-    slot_free, ready, n_px = [None, None], [None] * len(chunks), [0] * len(chunks)
+    push = _side_stream(device, "push")
 
-    def upload(ci):
-        v0 = chunks[ci]
-        with torch.cuda.stream(copy):
-            if slot_free[ci % 2] is not None:
-                copy.wait_event(slot_free[ci % 2])
-            n_px[ci] = _copy_views(seg_maps, sizes, v0, min(v0 + CH, v_hi), slots[ci % 2])
-            ready[ci] = torch.cuda.Event()
-            ready[ci].record(copy)
+    def push_chunk(v0, v1, packed):
+        """Push packed views [v0, v1) to every peer while the next chunk uploads."""
+        done = torch.cuda.Event()
+        done.record(main)
+        a, b = int(pstarts[v0]), int(pstarts[v1])
+        with torch.cuda.stream(push):
+            push.wait_event(done)
+            for k in range(1, world):
+                r = (rank + k) % world
+                peers[r][a:b].copy_(packed[a:b], non_blocking=True)
 
     with torch.cuda.device(device):
-        for ci in range(min(2, len(chunks))):
-            upload(ci)
-        if before_wait is not None:
-            before_wait()
-        minmax = torch.tensor([2**31 - 1, -2**31], dtype=torch.int32, device=device)
-        err = torch.zeros(1, dtype=torch.int32, device=device)
-        push = _push_stream(device)
-        for ci, v0 in enumerate(chunks):
-            v1 = min(v0 + CH, v_hi)
-            buf = slots[ci % 2]
-            main.wait_event(ready[ci])
-            check(L.gsl_label_range(buf.data_ptr(), n_px[ci], minmax.data_ptr(), main.cuda_stream))
-            for v, n in _runs(shapes, v0, v1):
-                check(L.gsl_pack_labels(buf.data_ptr() + 4 * int(starts[v] - starts[v0]), n, shapes[v][1], shapes[v][0],
-                                        packed.data_ptr() + int(pstarts[v]), -1, ops.DEFAULT_N_CLASSES, err.data_ptr(), main.cuda_stream))
-            slot_free[ci % 2] = torch.cuda.Event()
-            slot_free[ci % 2].record(main)
-            if ci + 2 < len(chunks):
-                upload(ci + 2)
-            if peers is not None:                    # push this chunk to every peer while the next one uploads
-                done = torch.cuda.Event()
-                done.record(main)
-                a, b = int(pstarts[v0]), int(pstarts[v1])
-                with torch.cuda.stream(push):
-                    push.wait_event(done)
-                    for k in range(1, world):
-                        r = (rank + k) % world
-                        peers[r][a:b].copy_(packed[a:b], non_blocking=True)
+        packed, minmax = _stage_int32(seg_maps, shapes, sizes, starts, pstarts, device, v_lo, v_hi, packed, before_wait,
+                                      push_chunk if peers is not None else None)
         mm = torch.stack([minmax[0].to(torch.int64), -minmax[1].to(torch.int64)])
         dist.all_reduce(mm, op=dist.ReduceOp.MIN)
         if peers is not None:
@@ -463,30 +438,8 @@ def _stage_sharded(seg_maps, shapes, device, dist, world, rank, before_wait=None
                 if b > a:
                     dist.broadcast(packed[a:b], src=r)
         lo, hi = int(mm[0].item()), -int(mm[1].item())
-    return _Staged(packed, -1, ops.DEFAULT_N_CLASSES, lo, hi, 4 * int(starts[v_hi] - starts[v_lo]), V, 0)
-
-
-_push_streams = {}
-
-
-def _push_stream(device):
-    key = (device.type, device.index)
-    if key not in _push_streams:
-        _push_streams[key] = torch.cuda.Stream(device)
-    return _push_streams[key]
-
-
-def _stage_wide(seg_maps, shapes, device):
-    """Label sets that do not fit one 254-code window (reference dls:288-295 accepts any int32
-    label): all maps go to the device as int32 and every value is replaced by its rank among the
-    distinct values (dense ids), which the caller then lifts in passes of 254 ids.  Returns
-    (dense int32 maps flat, sorted distinct values)."""
-    sizes = [h * w for h, w in shapes]
-    staged = torch.empty(int(sum(sizes)), dtype=torch.int32, device=device)
-    _copy_views(seg_maps, sizes, 0, len(seg_maps), staged)
-    uniq = torch.unique(staged)                                  # sorted
-    dense = torch.searchsorted(uniq, staged).to(torch.int32)
-    return dense, uniq
+    last_call_stats.update(h2d_bytes=4 * int(starts[v_hi] - starts[v_lo]), views_as_int32=V, views_narrowed_on_host=0)
+    return packed, lo, hi
 
 
 def lift_labels(positions, cameras, seg_maps, image_sizes=None, device=None, want_near=False,
@@ -498,7 +451,7 @@ def lift_labels(positions, cameras, seg_maps, image_sizes=None, device=None, wan
     seg_maps    list of int arrays [seg_h, seg_w] (NumPy or tensors), one per camera; any int32
                 label values (more than 254 distinct values are lifted in several passes)
     image_sizes per camera (orig_w, orig_h); default = the map's own size (scale 1.0)
-    label_min, n_classes  optional explicit code window (values outside it raise)
+    label_min, n_classes  optional explicit code window, both or neither (values outside it raise)
     Returns int32 NumPy labels (and the near-boundary mask when want_near).
     """
     from ._native import check, lib
@@ -510,6 +463,8 @@ def lift_labels(positions, cameras, seg_maps, image_sizes=None, device=None, wan
     shapes = [tuple(int(x) for x in m.shape) for m in seg_maps]
     if any(len(sh) != 2 for sh in shapes):
         raise ValueError("every segmentation map must be 2-D [seg_h, seg_w]")
+    if (label_min is None) != (n_classes is None):
+        raise ValueError("give both label_min and n_classes, or neither")
     dist, world, rank = _dist()
     V = len(cameras)
     if len(seg_maps) != V:
@@ -530,52 +485,58 @@ def lift_labels(positions, cameras, seg_maps, image_sizes=None, device=None, wan
             check(L.gsl_lift_prepare(pos.data_ptr(), N, views.ctypes.data, V, ws.data_ptr(), ws.numel(), main.cuda_stream))
         state.update(pos=pos, views=views, N=N, ws=ws)
 
+    def gather(packed, v0, v1):
+        with torch.cuda.device(device):
+            check(L.gsl_lift_gather_range(state["pos"].data_ptr(), state["N"], state["views"].ctypes.data, V, v0, v1,
+                                          packed.data_ptr(), state["ws"].data_ptr(), state["ws"].numel(), main.cuda_stream))
+
     def sweep(packed, lmin, ncls, best=None, v_from=0):
         """Gather views [v_from, V) (earlier ones were swept while the maps were uploading), then the majority."""
         labels = torch.empty(state["N"], dtype=torch.int32, device=device)
-        a = (state["pos"].data_ptr(), state["N"], state["views"].ctypes.data, V)
-        w = (state["ws"].data_ptr(), state["ws"].numel(), main.cuda_stream)
+        gather(packed, v_from, V)
         with torch.cuda.device(device):
-            check(L.gsl_lift_gather_range(*a, int(v_from), V, packed.data_ptr(), *w))
             check(L.gsl_lift_majority(state["N"], V, int(lmin), int(ncls), labels.data_ptr(),
-                                      best.data_ptr() if best is not None else None, *w))
+                                      best.data_ptr() if best is not None else None,
+                                      state["ws"].data_ptr(), state["ws"].numel(), main.cuda_stream))
         return labels
 
     swept = [0]
 
-    def sweep_resident(v_done, packed):
-        """Staging callback: views [0, v_done) are packed (enqueued on the main stream); sweep the
+    def sweep_resident(v0, v1, packed):
+        """Staging callback: views [0, v1) are packed (enqueued on the main stream); gather the
         complete groups of 32 among them -- a sweep CTA takes two 16-view windows."""
-        target = v_done if v_done == V else v_done // 32 * 32
+        target = v1 if v1 == V else v1 // 32 * 32
         if target > swept[0]:
-            with torch.cuda.device(device):
-                check(L.gsl_lift_gather_range(state["pos"].data_ptr(), state["N"], state["views"].ctypes.data, V, swept[0], target,
-                                              packed.data_ptr(), state["ws"].data_ptr(), state["ws"].numel(), main.cuda_stream))
+            gather(packed, swept[0], target)
             swept[0] = target
 
     if V == 0 or positions.shape[0] == 0:
         labels = np.full(positions.shape[0], -1, dtype=np.int32)
         return (labels, np.zeros(positions.shape[0], np.uint8)) if want_near else labels
 
+    lmin, ncls = ops.DEFAULT_LABEL_MIN, ops.DEFAULT_N_CLASSES
     wide = False
-    if label_min is not None and n_classes is not None:
+    if label_min is not None:
+        lmin, ncls = int(label_min), int(n_classes)
         prepare()
-        packed = _pack_explicit(seg_maps, shapes, device, int(label_min), int(n_classes))
-        st = _Staged(packed, int(label_min), int(n_classes), int(label_min), int(label_min) + int(n_classes) - 1,
-                     4 * sum(h * w for h, w in shapes), V, 0)
-    elif world > 1:
-        st = _stage_sharded(seg_maps, shapes, device, dist, world, rank, before_wait=prepare)
+        staged = _upload_all(seg_maps, shapes, device)
+        packed = ops.pack_labels(staged, shapes, lmin, ncls)              # raises on a value outside the window
+        last_call_stats.update(h2d_bytes=4 * staged.numel(), views_as_int32=V, views_narrowed_on_host=0)
     else:
-        st = _stage_pipelined(seg_maps, shapes, device, before_wait=prepare, on_packed=sweep_resident)
-    if st.lo < st.label_min or st.hi > st.label_min + st.n_classes - 1:
-        if label_min is not None and n_classes is not None:
-            raise ValueError(f"label map value outside [{label_min}, {label_min + n_classes})")
-        wide = True
+        if world > 1:
+            packed, lo, hi = _stage_sharded(seg_maps, shapes, device, dist, world, rank, prepare)
+        else:
+            packed, lo, hi = _stage_single(seg_maps, shapes, device, prepare, sweep_resident)
+        wide = lo < lmin or hi > lmin + ncls - 1
+        ncls = min(max(hi - lmin + 1, 1), ncls) if hi >= lo else 1      # fewer histogram rows per Gaussian
     if not wide:
-        ncls = max(st.hi - st.label_min + 1, 1) if st.hi >= st.lo else 1      # fewer histogram rows per Gaussian
-        labels = sweep(st.packed, st.label_min, min(ncls, st.n_classes), v_from=swept[0])
+        labels = sweep(packed, lmin, ncls, v_from=swept[0])
+        n_passes = 1
     else:
-        dense, uniq = _stage_wide(seg_maps, shapes, device)
+        staged = _upload_all(seg_maps, shapes, device)
+        last_call_stats["h2d_bytes"] += 4 * staged.numel()
+        uniq = torch.unique(staged)                                     # sorted
+        dense = torch.searchsorted(uniq, staged).to(torch.int32)        # every value -> its rank among the distinct values
         n_ids = int(uniq.numel())
         labels = best = None
         packed = torch.empty(int(ops.packed_offsets(shapes)[-1]), dtype=torch.uint8, device=device)
@@ -591,27 +552,18 @@ def lift_labels(positions, cameras, seg_maps, image_sizes=None, device=None, wan
                 ops.lift_merge(labels, best, lab, b)
         seen = labels >= 0
         labels = torch.where(seen, uniq[labels.clamp(min=0).long()], labels)           # dense id -> the map's own value
-        st.h2d_bytes = 4 * sum(h * w for h, w in shapes) + st.h2d_bytes
-    last_call_stats.update(h2d_bytes=st.h2d_bytes + int(state["pos"].numel()) * 4, d2h_bytes=int(state["N"]) * 4,
-                           views_as_int32=st.views_as_int32, views_narrowed_on_host=st.views_narrowed,
-                           label_passes=1 if not wide else -(-n_ids // ops.DEFAULT_N_CLASSES))
+        n_passes = -(-n_ids // P)
+    last_call_stats.update(h2d_bytes=last_call_stats["h2d_bytes"] + int(state["pos"].numel()) * 4,
+                           d2h_bytes=int(state["N"]) * 4, label_passes=n_passes)
     if trace:
         torch.cuda.synchronize(device)
         print(f"[gslift trace] lift_labels: staging + sweep {1e3 * (time.perf_counter() - t_enter):.2f} ms, "
-              f"{st.views_as_int32} views as int32, {st.views_narrowed} narrowed on the host", file=sys.stderr)
+              f"{last_call_stats['views_as_int32']} views as int32, {last_call_stats['views_narrowed_on_host']} narrowed on the host",
+              file=sys.stderr)
     if want_near:
         near = ops.lift_near(state["pos"], state["views"], near_eps)
         return _to_host(labels), _to_host(near)
     return _to_host(labels)
-
-
-def _pack_explicit(seg_maps, shapes, device, label_min, n_classes):
-    """Upload every map as int32 and pack it with the caller's code window (raises on a value
-    outside it)."""
-    sizes = [h * w for h, w in shapes]
-    staged = torch.empty(int(sum(sizes)), dtype=torch.int32, device=device)
-    _copy_views(seg_maps, sizes, 0, len(seg_maps), staged)
-    return ops.pack_labels(staged, shapes, label_min, n_classes)
 
 
 def _to_host(t: torch.Tensor) -> np.ndarray:

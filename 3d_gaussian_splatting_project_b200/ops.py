@@ -99,6 +99,17 @@ def make_views(cameras, map_shapes, image_sizes=None) -> np.ndarray:
     return views
 
 
+def _runs(shapes, v0, v1):
+    """(first view, count) of the runs of equal map shapes among views [v0, v1): one pack launch each."""
+    v = v0
+    while v < v1:
+        n = 1
+        while v + n < v1 and shapes[v + n] == shapes[v]:
+            n += 1
+        yield v, n
+        v += n
+
+
 def pack_labels(maps: torch.Tensor, shapes=None, label_min: int = DEFAULT_LABEL_MIN,
                 n_classes: int = DEFAULT_N_CLASSES, out: torch.Tensor | None = None,
                 check_range: bool = True) -> torch.Tensor:
@@ -130,16 +141,12 @@ def pack_labels(maps: torch.Tensor, shapes=None, label_min: int = DEFAULT_LABEL_
     flat = maps.reshape(-1)
     L = lib()
     with torch.cuda.device(maps.device):
-        v, src = 0, 0
-        while v < len(shapes):                       # one launch per run of equal shapes
-            n = 1
-            while v + n < len(shapes) and shapes[v + n] == shapes[v]:
-                n += 1
+        src = 0
+        for v, n in _runs(shapes, 0, len(shapes)):
             h, w = shapes[v]
             check(L.gsl_pack_labels(flat.data_ptr() + 4 * src, n, w, h, out.data_ptr() + int(offs[v]),
                                     int(label_min), int(n_classes), err.data_ptr(), _stream()))
             src += n * h * w
-            v += n
     if check_range and int(err.item()) != 0:
         raise ValueError(f"label map value outside [{label_min}, {label_min + n_classes})")
     return out

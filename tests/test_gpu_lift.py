@@ -208,6 +208,12 @@ def test_empty_inputs_and_label_range():
     got = dls.lift_labels(pos, cams, shifted)
     ref = dls.lift_labels(pos, cams, maps0)
     assert (ref >= 0).any() and np.array_equal(np.where(ref == -1, -1, ref + 1000), got)
+    # no Gaussians, or no views, through lift_labels: -1 labels of the right length, a zero mask
+    for p, cc, mm in ((pos[:0], cams, list(maps)), (pos, [], [])):
+        labels = dls.lift_labels(p, cc, mm)
+        assert labels.dtype == np.int32 and labels.shape == (len(p),) and (labels == -1).all()
+        labels, near = dls.lift_labels(p, cc, mm, want_near=True)
+        assert labels.shape == near.shape == (len(p),) and (labels == -1).all() and not near.any()
 
 
 def test_full_size_c3_properties_and_oracle(oracle):
@@ -327,6 +333,56 @@ def test_hybrid_staging_host_narrowed_views_give_the_same_labels(oracle, monkeyp
     monkeypatch.setenv("GSLIFT_HOST_STAGE", fraction)
     got = dls.lift_labels(pos, cams, maps, sizes)
     compare(got, want)
+
+
+@pytest.mark.parametrize("fraction", ["0", "0.5"])
+def test_lift_labels_from_rows_of_one_pinned_tensor(oracle, monkeypatch, fraction):
+    """The benchmark's call: pinned CPU positions, maps as rows of one pinned int32 tensor (they
+    cross in coalesced copies), 48 views = three 16-view chunks, so that with a host share of 0.5
+    one chunk crosses as int32 and two are narrowed on the host.  The byte counts of
+    last_call_stats follow the split."""
+    dls = pkg("deep_learning_segmentation")
+    v, w, h = 48, 320, 200
+    cams, pos, maps = _scene(30_000, v, w, h, seed=91)
+    want, _, _ = oracle.lift_votes(pos, oracle.make_views(cams, [(h, w)] * v), maps)
+    rows = torch.from_numpy(maps).pin_memory()
+    monkeypatch.setenv("GSLIFT_HOST_STAGE", fraction)
+    got = dls.lift_labels(torch.from_numpy(pos).pin_memory(), cams, [rows[i] for i in range(v)], None, device=DEV)
+    compare(got, want)
+    st = dls.last_call_stats
+    as_int32, narrowed = st["views_as_int32"], st["views_narrowed_on_host"]
+    assert as_int32 + narrowed == v and (as_int32, narrowed) == ((v, 0) if fraction == "0" else (16, 32))
+    assert st["h2d_bytes"] == 4 * as_int32 * h * w + narrowed * h * w + 12 * len(pos)
+    assert st["d2h_bytes"] == 4 * len(pos) and st["label_passes"] == 1
+
+
+def test_lift_labels_explicit_code_window(oracle):
+    """label_min and n_classes given together: the maps are packed with that window and the labels
+    are the oracle's; a map value outside the window raises, and so does giving only one of the two."""
+    dls = pkg("deep_learning_segmentation")
+    v, w, h = 20, 320, 200
+    cams, pos, maps = _scene(20_000, v, w, h, seed=81)
+    want, _, _ = oracle.lift_votes(pos, oracle.make_views(cams, [(h, w)] * v), maps)
+    compare(dls.lift_labels(pos, cams, list(maps), label_min=-1, n_classes=151), want)
+    for bad_value in (150, -2):
+        bad = maps.copy()
+        bad[17, 5, 9] = bad_value
+        with pytest.raises(ValueError, match="outside"):
+            dls.lift_labels(pos, cams, list(bad), label_min=-1, n_classes=151)
+    for half in ({"label_min": -1}, {"n_classes": 151}):
+        with pytest.raises(ValueError, match="label_min and n_classes"):
+            dls.lift_labels(pos, cams, list(maps), **half)
+
+
+def test_lift_labels_want_near_equals_lift_votes():
+    """want_near=True through lift_labels: labels and near-boundary mask of ops.lift_votes."""
+    dls = pkg("deep_learning_segmentation")
+    cams, pos, maps = _scene(40_000, 21, 320, 200, seed=83)
+    labels, near = dls.lift_labels(pos, cams, list(maps), want_near=True, near_eps=1e-4)
+    want, want_near = gpu_lift(pos, cams, list(maps), None, want_near=True, near_eps=1e-4)
+    assert labels.dtype == np.int32 and near.dtype == np.uint8
+    assert np.array_equal(labels, want.cpu().numpy()) and np.array_equal(near, want_near.cpu().numpy())
+    assert near.any()
 
 
 def test_more_than_255_distinct_labels(oracle):

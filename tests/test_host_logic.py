@@ -142,6 +142,33 @@ def test_slice_bounds_partition():
             assert max(sizes) - min(sizes) <= 1
 
 
+def test_lift_labels_staging_plan():
+    """The one-process staging plan of lift_labels: views [0, v_int32) cross as int32, the host
+    narrows the rest in batches of two 16-view chunks while more than three chunks remain, then one
+    chunk at a time; every view is staged once, in order, and the bytes on the bus follow the split."""
+    plan, CH = pkg("deep_learning_segmentation")._chunk_plan, 16
+    px = 1080 * 1920                                     # the benchmark: 300 views of 1920 x 1080
+    assert plan([(1080, 1920)] * 300, 0.4) == (176, [(176, 208), (208, 240), (240, 272), (272, 288), (288, 300)],
+                                                4 * 176 * px + 124 * px)
+    assert plan([(1080, 1920)] * 300, 0.0) == (300, [], 4 * 300 * px)
+    assert plan([(200, 320)] * 48, 0.5) == (16, [(16, 32), (32, 48)], (4 * 16 + 32) * 200 * 320)
+    for V in (1, 15, 16, 17, 33, 48, 63, 64, 65, 300, 401):
+        shapes = [(7 + v % 5, 11 + v % 3) for v in range(V)]
+        sizes = [h * w for h, w in shapes]
+        n_chunks = -(-V // CH)
+        for f in (0.0, 0.1, 0.25, 0.4, 0.5, 0.85, 1.0):
+            v_int32, batches, nbytes = plan(shapes, f)
+            assert v_int32 == min((n_chunks - round(f * n_chunks)) * CH, V)
+            ranges = [(0, v_int32)] + batches
+            assert [a for a, _ in ranges[1:]] == [b for _, b in ranges[:-1]] and ranges[-1][1] == V   # once, in order
+            assert all(a % CH == 0 and a < b for a, b in batches)
+            per_batch = [-(-(b - a) // CH) for a, b in batches]                                     # chunks per batch
+            m = n_chunks - v_int32 // CH if batches else 0
+            k = max(0, (m - 2) // 2)
+            assert per_batch == [2] * k + [1] * (m - 2 * k)
+            assert nbytes == 4 * sum(sizes[:v_int32]) + sum(sizes[v_int32:])
+
+
 _WORKER = r'''
 import os, sys, importlib
 import numpy as np, torch, torch.distributed as dist
