@@ -221,8 +221,8 @@ def lift_phases(pos: torch.Tensor, views: np.ndarray, packed: torch.Tensor,
     zero-argument callables that enqueue gsl_lift_prepare (ordering + per-tile verdicts; reads no
     maps), gsl_lift_gather (projection + visibility + gather into the vote sheet) and
     gsl_lift_majority on the current stream (benchmarks put events between them); run_sweep is
-    gsl_lift_sweep = gather + majority with the majority of one chunk of Gaussians overlapping the
-    sweep of the next (what lift_votes runs)."""
+    gsl_lift_sweep = the gather over all Gaussians, then the majority over all of them, back to back
+    on the same stream (the two steps lift_votes runs after the prepare step)."""
     views = _check_lift(pos, views, packed)
     N, V = pos.shape[0], len(views)
     labels = out if out is not None else torch.empty(N, dtype=torch.int32, device=pos.device)
